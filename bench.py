@@ -93,12 +93,11 @@ def usable_cores():
 # ------------------------------------------------------------- CPU baselines
 
 def reference_root():
-  """Directory holding the UNMODIFIED reference package, if any travelled here:
-  the driver's / builder's offline install `baseline/_ref` (pip --target, git-ignored,
-  ships with the snapshot), else the read-only checkout of the build container."""
-  for root in (os.path.join(ROOT, 'baseline', '_ref'), '/root/reference'):
-    if os.path.isfile(os.path.join(root, 'pycolab', 'engine.py')):
-      return root
+  """Directory holding the UNMODIFIED reference package, if an offline install of it
+  (`pip install --target baseline/_ref`, git-ignored) sits beside this file."""
+  root = os.path.join(ROOT, 'baseline', '_ref')
+  if os.path.isfile(os.path.join(root, 'pycolab', 'engine.py')):
+    return root
   return None
 
 
@@ -744,7 +743,11 @@ def main():
                   help='skip the C3/C4/C5 block (headline only)')
   ap.add_argument('--levels', default='shared', choices=['shared', 'per-env'],
                   help='static level data: one copy per level (default) or one per env')
+  ap.add_argument('--dump-outputs', metavar='DIR',
+                  help='write what the last timed step returned (rank 0) as DIR/<name>.npy')
   args = ap.parse_args()
+  if args.dump_outputs and args.impl == 'reference':
+    ap.error('--dump-outputs writes what the device step returned; --impl reference has none')
 
   rank = int(os.environ.get('RANK', '0'))
   world = int(os.environ.get('WORLD_SIZE', '1'))
@@ -814,6 +817,8 @@ def main():
   l_before = sum(e.launch_count() for e in engines)
   dev_ms_local = timed.time_ms(barrier)
   wall = time.perf_counter() - wall0
+  if args.dump_outputs and rank == 0:
+    dump_outputs(args.dump_outputs, engines[(W + K - 1) % R])
   launches = K if timed.graphs else sum(e.launch_count() for e in engines) - l_before
   dev_ms, per_rank_ms = max_over_ranks(torch, dist, dev, world, dev_ms_local)
   value = world * B * K / (dev_ms / 1000.0)
@@ -990,6 +995,23 @@ def main():
     real_stdout.flush()
   if world > 1:
     dist.destroy_process_group()
+
+
+DUMP_BOARDS = 1024                # envs whose boards --dump-outputs writes (16 MB as f32)
+
+
+def dump_outputs(path, eng):
+  """The StepResult of `eng`'s last step as float32 .npy files: reward, has_reward,
+  discount and done of every env, and the boards of a fixed, seeded sample of
+  DUMP_BOARDS envs (all B boards as float32 would be 64 MB) with their indices."""
+  os.makedirs(path, exist_ok=True)
+  envs = np.sort(np.random.RandomState(0).choice(eng.batch, min(DUMP_BOARDS, eng.batch),
+                                                 replace=False))
+  arrays = {'board_sample': eng.board.cpu().numpy()[envs], 'board_sample_env': envs,
+            'reward': eng.reward.cpu().numpy(), 'has_reward': eng.has_reward.cpu().numpy(),
+            'discount': eng.discount.cpu().numpy(), 'done': eng.done.cpu().numpy()}
+  for name, a in arrays.items():
+    np.save(os.path.join(path, name + '.npy'), a.astype(np.float32))
 
 
 def per_env_level_point(torch, dist, dev, world, rank, lowered, actions, W, K, barrier, peak):

@@ -194,7 +194,7 @@ class Tracker(unittest.TextTestResult):
 
 
 def main():
-  assert refdriver.available(), '/root/reference is required'
+  assert refdriver.available(), refdriver.MISSING
   install()
   suite = unittest.defaultTestLoader.loadTestsFromModule(engine_test)
   result = unittest.TextTestRunner(verbosity=1, resultclass=Tracker).run(suite)

@@ -1,6 +1,6 @@
 """Generate the golden fixtures in this directory from the REAL reference.
 
-Run in the build container (where /root/reference exists):
+Run with PYCOLAB_UPSTREAM naming an upstream pycolab checkout:
 
     python tests/golden/make_golden.py
 
@@ -539,7 +539,7 @@ def classic(name, kind, art, actions):
 
 
 def main():
-  assert refdriver.available(), '/root/reference is required'
+  assert refdriver.available(), refdriver.MISSING
   if sys.argv[1:] == ['classics']:      # add these without rewriting the older files
     return classics()
   if sys.argv[1:] == ['stories']:

@@ -1,6 +1,6 @@
 """Capture the reference's OWN known-answer tests as replayable fixtures.
 
-Run in the build container (where /root/reference exists):
+Run with PYCOLAB_UPSTREAM naming an upstream pycolab checkout:
 
     python tests/golden/make_kats.py
 
@@ -184,7 +184,7 @@ def numpy2_shim():
 
 
 def main():
-  assert refdriver.available(), '/root/reference is required'
+  assert refdriver.available(), refdriver.MISSING
   tt.PycolabTestCase.assertMachinima = capture
   real_assert = numpy2_shim()
   suite = unittest.TestSuite()

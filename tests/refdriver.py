@@ -1,9 +1,9 @@
-"""Drive the REAL reference (imported from /root/reference) on arbitrary art.
+"""Drive the original pycolab (an upstream checkout) on arbitrary art.
 
-Only usable where /root/reference exists (this build container); used by
-`tests/golden/make_golden.py` to produce the committed golden fixtures and by
-`tests/test_oracle_vs_reference.py` for live differential checks.  Never
-imported on the GPU box.
+Set PYCOLAB_UPSTREAM to the directory that holds the upstream `pycolab` package.
+The generators under `tests/golden/` use it to produce the committed golden
+fixtures; the one test that runs an upstream example file itself on the device
+skips without it.  Nothing else in the suite needs it.
 """
 
 import os
@@ -11,11 +11,12 @@ import sys
 
 import numpy as np
 
-REFERENCE_ROOT = '/root/reference'
+REFERENCE_ROOT = os.environ.get('PYCOLAB_UPSTREAM', '')
+MISSING = 'needs an upstream pycolab checkout (set PYCOLAB_UPSTREAM)'
 
 
 def available():
-  return os.path.isdir(os.path.join(REFERENCE_ROOT, 'pycolab'))
+  return bool(REFERENCE_ROOT) and os.path.isdir(os.path.join(REFERENCE_ROOT, 'pycolab'))
 
 
 def _import():
@@ -248,3 +249,95 @@ def snapshot_things(engine):
     if hasattr(ent, 'position'):
       out[ch] = (int(ent.position[0]), int(ent.position[1]), bool(ent.visible))
   return out
+
+
+def _result_code(result):
+  """A MazeWalker motion result in the oracle's encoding (engine_model.EDGE)."""
+  from oracle import engine_model as em
+  def code(x):
+    return em.EDGE if x == 'edge!' else ord(x)
+  if result is None:
+    return None
+  if isinstance(result, tuple):
+    return tuple(code(x) for x in result)
+  return code(result)
+
+
+class ReferenceSide(object):
+  """The original's engines for the scenarios of tests/reference_trace.py."""
+
+  def scrolly_stock(self, level):
+    return lambda: ref_scrolly_maze(None, None, level=level)
+
+  def scrolly(self, maze, board, beneath):
+    return lambda: ref_scrolly_maze(maze, board, beneath)
+
+  def warehouse_stock(self, level):
+    return lambda: ref_warehouse(None, level=level)
+
+  def warehouse(self, art, beneath):
+    return lambda: ref_warehouse(art, beneath)
+
+  def marauders(self, seed):
+    np.random.seed(seed)                  # the original draws from the global RNG
+    return ref_marauders
+
+  def fixture(self, art, walkers, scrollys=None, **kw):
+    return ref_fixture(art, ' ', walkers, scrollys, **kw)
+
+  def fixture_action(self, action):
+    return fixture_actions_to_ref(action)
+
+  def walk_result(self, engine, ch):
+    return _result_code(engine.the_plot['walk_result_' + ch])
+
+  def classic(self, kind, art):
+    return lambda: ref_classic(kind, art)
+
+  def aperture(self, level, art):
+    return lambda: ref_aperture(level, art)
+
+  def fluvial(self, art):
+    art = art or ref_fluvial_art()
+    return lambda: ref_fluvial(art)
+
+  def scrolly_cropper(self, engine, pad, margins):
+    crop = _import()['cropping'].ScrollingCropper(rows=9, cols=9, to_track=['P'],
+                                                  scroll_margins=margins, pad_char=pad)
+    crop.set_engine(engine)
+    return lambda out: crop.crop(out[0]).board
+
+  def ordeal(self):
+    ref_storytelling()
+    from pycolab.examples import ordeal
+    return ordeal.make_game()
+
+  def ordeal_chapter(self, story):
+    return story.the_plot.this_chapter
+
+  def apprehend(self, seed):
+    import random
+    _import()
+    from pycolab.examples import apprehend
+    random.seed(seed)
+    return apprehend.make_game()
+
+  def ball_registers(self, engine):
+    ball = engine.things['b']
+    return float(ball._dx), float(ball._x_accumulator)
+
+  def shockwave(self, art, seed):
+    _import()
+    from pycolab.examples import shockwave as m
+    np.random.seed(seed)
+    saved = m.LEVELS
+    try:
+      m.LEVELS = [art]
+      return m.make_game(0)
+    finally:
+      m.LEVELS = saved
+
+  def shockwave_stock_art(self):
+    _import()
+    from pycolab.examples import shockwave as m
+    return m.LEVELS[0]

@@ -11,7 +11,7 @@ import numpy as np
 import pytest
 
 import golden_cases as gc
-import refdriver
+import reference_trace as rt
 import trajectory as tj
 from oracle import games as ogames
 
@@ -131,23 +131,10 @@ def test_apprehend_lowers_and_validates_on_cpu():
   assert lib.pcl_create(C.byref(spec), 4, -1, C.byref(handle)) != _lib.OK
 
 
-@pytest.mark.skipif(not refdriver.available(), reason='/root/reference not present')
 def test_reference_apprehend_file_lowers_like_the_twin():
-  import sys
-  from pycolab_b200 import compat, lowering
+  """The original's examples/apprehend.py, loaded through `compat` with
+  random.seed(11), lowered to what this package's twin lowers to."""
+  from pycolab_b200 import lowering
   from pycolab_b200.games import apprehend
-  saved = {k: v for k, v in sys.modules.items() if k == 'pycolab' or k.startswith('pycolab.')}
-  compat.uninstall()
-  try:
-    mod = compat.load_example(os.path.join(refdriver.REFERENCE_ROOT, 'pycolab', 'examples',
-                                           'apprehend.py'))
-    random.seed(11)
-    a = lowering.lower(mod.make_game())
-    random.seed(11)
-    b = lowering.lower(apprehend.make_game())
-    assert a.signature() == b.signature()
-    for field in ('backdrop', 'sprites', 'drapes', 'plot'):
-      np.testing.assert_array_equal(getattr(a, field), getattr(b, field), err_msg=field)
-  finally:
-    compat.uninstall()
-    sys.modules.update(saved)
+  random.seed(11)
+  rt.check_lowering('apprehend', lowering.lower(apprehend.make_game()))

@@ -8,7 +8,7 @@ import numpy as np
 import pytest
 
 import golden_cases as gc
-import refdriver
+import reference_trace as rt
 import trajectory as tj
 from oracle import games as ogames
 
@@ -94,21 +94,11 @@ def test_batched_hello_vs_oracle():
   assert int(eng.error_codes().abs().max()) == 0
 
 
-@pytest.mark.skipif(not refdriver.available(), reason='/root/reference not present')
 def test_reference_hello_world_file_lowers_like_the_twin():
-  import sys
-  from pycolab_b200 import compat, lowering
+  """The original's examples/hello_world.py, loaded through `compat`, lowered to
+  what this package's twin lowers to."""
+  from pycolab_b200 import lowering
   from pycolab_b200.games import hello_world
-  saved = {k: v for k, v in sys.modules.items() if k == 'pycolab' or k.startswith('pycolab.')}
-  compat.uninstall()
-  try:
-    mod = compat.load_example(os.path.join(refdriver.REFERENCE_ROOT, 'pycolab', 'examples',
-                                           'hello_world.py'))
-    a, b = lowering.lower(mod.make_game()), lowering.lower(hello_world.make_game())
-    assert a.signature() == b.signature()
-    for field in ('backdrop', 'sprites', 'drapes', 'plot'):
-      np.testing.assert_array_equal(getattr(a, field), getattr(b, field), err_msg=field)
-    np.testing.assert_array_equal(a.bits[0], b.bits[0])
-  finally:
-    compat.uninstall()
-    sys.modules.update(saved)
+  with rt.sorted_default_schedule():
+    game = hello_world.make_game()
+  rt.check_lowering('hello_world', lowering.lower(game))

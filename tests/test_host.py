@@ -1,5 +1,5 @@
 """CPU tests of the host side: C-ABI library surface, facade set-up API,
-lowering, compat loading of the reference's example modules."""
+lowering, compat loading of example modules."""
 
 import os
 import sys
@@ -9,7 +9,7 @@ import numpy as np
 import pytest
 
 import golden_cases as gc
-import refdriver
+import reference_trace as rt
 import trajectory as tj
 from oracle import games as ogames
 from pycolab_b200 import _lib
@@ -318,221 +318,279 @@ def test_maze_walker_constructor_contract():
   assert bolt.position == (3, 1) and bolt.visible
 
 
-# --------------------------------- the reference's own example files, unchanged
-
-needs_ref = pytest.mark.skipif(not refdriver.available(),
-                               reason='/root/reference not present')
-
+# ------------------- the original's example files, as they lower through compat
+# tests/golden/reference_lowerings.json holds a digest of what each of the
+# original's example files lowered to when loaded unmodified through `compat`
+# (tests/golden/make_reference_traces.py); this package's twins must lower to
+# exactly that.
 
 @pytest.fixture
-def compat_examples():
-  import sys
+def compat_loader(tmp_path):
+  """Writes a module source into tmp_path and loads it through `compat`, the way
+  a user's copy of an example file is loaded."""
   from pycolab_b200 import compat
   saved = {k: v for k, v in sys.modules.items()
            if k == 'pycolab' or k.startswith('pycolab.')}
   compat.uninstall()
   compat.install()
-  base = os.path.join(refdriver.REFERENCE_ROOT, 'pycolab', 'examples')
-  yield lambda name: compat.load_example(os.path.join(base, name + '.py'))
+
+  def load(name, source, copy='a'):
+    path = tmp_path / copy / (name + '.py')
+    path.parent.mkdir(exist_ok=True)
+    path.write_text(source)
+    return compat.load_example(str(path))
+  yield load
   compat.uninstall()
   sys.modules.update(saved)
 
 
-def _same_lowering(a, b):
-  assert a.signature() == b.signature()
-  for name in ('backdrop', 'sprites', 'drapes', 'plot'):
-    np.testing.assert_array_equal(getattr(a, name), getattr(b, name), err_msg=name)
-  for d in a.patterns:
-    np.testing.assert_array_equal(a.patterns[d], b.patterns[d])
-  for d in a.bits:
-    np.testing.assert_array_equal(a.bits[d], b.bits[d])
-
-
-@needs_ref
-def test_reference_scrolly_maze_example_loads_and_lowers(compat_examples):
-  mod = compat_examples('scrolly_maze')
-  assert mod.PlayerSprite.__mro__[1] is prefab_sprites.MazeWalker
+def test_reference_scrolly_maze_example_loads_and_lowers():
   for level in (0, 1, 2):
-    theirs = lowering.lower(mod.make_game(level))
-    ours = lowering.lower(g_scrolly.make_game(
-        mod.MAZES_ART[level], mod.STAR_ART, mod.MAZES_WHAT_LIES_BENEATH[level]))
-    _same_lowering(theirs, ours)
+    maze, board, beneath = gc.scrolly_art(gc.load('scrolly_stock_L%d' % level))
+    rt.check_lowering('scrolly_maze_%d' % level,
+                      lowering.lower(g_scrolly.make_game(maze, board, beneath)))
 
 
-@needs_ref
-def test_edited_copy_of_an_example_is_refused_not_replaced(compat_examples, tmp_path):
-  """A user's copy of scrolly_maze.py lowers while it is token-for-token the
-  reference's; with an edited update() (reward 7 instead of 100) the class is
-  named like a lowered class but is NOT that class: NotLoweredError, never the
-  stock kernel (lowering._is_known_implementation)."""
-  from pycolab_b200 import compat
-  from pycolab_b200.errors import NotLoweredError
-  src = open(os.path.join(refdriver.REFERENCE_ROOT, 'pycolab', 'examples',
-                          'scrolly_maze.py')).read()
-  same = tmp_path / 'same' / 'scrolly_maze.py'
-  same.parent.mkdir()
-  same.write_text('# my copy\n' + src.replace('\n\n', '\n\n\n', 1))   # comments/blank lines only
-  lowering.lower(compat.load_example(str(same)).make_game(0))
-  assert 'the_plot.add_reward(100)' in src
-  edited = tmp_path / 'edited' / 'scrolly_maze.py'
-  edited.parent.mkdir()
-  edited.write_text(src.replace('the_plot.add_reward(100)', 'the_plot.add_reward(7)'))
+def _user_copy_of_the_scrolly_maze_twin():
+  """This package's scrolly_maze set-up as a user's module: imports through the
+  `pycolab` alias, so its classes are not trusted by module."""
+  import inspect
+  return inspect.getsource(g_scrolly).replace('from pycolab_b200 import', 'from pycolab import') \
+      .replace('from pycolab_b200.prefab_parts', 'from pycolab.prefab_parts')
+
+
+def test_edited_copy_of_an_example_is_refused_not_replaced(compat_loader, monkeypatch):
+  """A user's copy of scrolly_maze.py lowers while its classes are token-for-token
+  the known implementation; with an edited class body the class is named like a
+  lowered class but is NOT that class: NotLoweredError, never the stock kernel
+  (lowering._is_known_implementation).  The known fingerprints are those of the
+  original's classes; here they are pointed at the copy's own classes."""
+  import inspect
+  from pycolab_b200 import _fingerprints
+  maze, board, beneath = gc.scrolly_art(gc.load('scrolly_stock_L0'))
+  src = _user_copy_of_the_scrolly_maze_twin()
+  mod = compat_loader('scrolly_maze', src)
+  assert mod.PlayerSprite.__mro__[1] is prefab_sprites.MazeWalker   # `pycolab` is this package
   with pytest.raises(NotLoweredError, match='source differs'):
-    lowering.lower(compat.load_example(str(edited)).make_game(0))
+    lowering.lower(mod.make_game(maze, board, beneath))     # not the original's source
+  for name in ('PlayerSprite', 'PatrollerSprite', 'MazeDrape', 'CashDrape'):
+    monkeypatch.setitem(_fingerprints.KNOWN, ('scrolly_maze', name),
+                        lowering.source_fingerprint(inspect.getsource(getattr(mod, name))))
+  same = compat_loader('scrolly_maze', '# my copy\n' + src.replace('\n\n', '\n\n\n', 1)
+                       .replace('\nclass PlayerSprite', '\n# the explorer\nclass PlayerSprite'),
+                       copy='same')
+  rt.check_lowering('scrolly_maze_0', lowering.lower(same.make_game(maze, board, beneath)))
+  assert "impassable='#')" in src
+  edited = compat_loader('scrolly_maze', src.replace("impassable='#')", "impassable='#@')", 1),
+                         copy='edited')
+  with pytest.raises(NotLoweredError, match='source differs'):
+    lowering.lower(edited.make_game(maze, board, beneath))
 
 
-@needs_ref
-def test_reference_warehouse_example_loads_and_lowers(compat_examples):
-  mod = compat_examples('warehouse_manager')
+_FINGERPRINTED = '''class PlayerSprite(prefab_sprites.MazeWalker):
+  """A walker that goes north on action 0 and stays put otherwise."""
+
+  def update(self, actions, board, layers, backdrop, things, the_plot):
+    del backdrop, things  # unused
+    if actions == 0:
+      self._north(board, the_plot)
+    else:
+      self._stay(board, the_plot)
+'''
+
+
+def test_source_fingerprint_normalisation_is_pinned():
+  """_fingerprints.KNOWN holds source_fingerprint() of the original's classes, so
+  the normalisation must not drift: a change to it would refuse every user's
+  unmodified example file.  Comments, blank lines, indentation width and an
+  enclosing indent do not count; any token does."""
+  import textwrap
+  want = '231bf765e8f4715d643edcbd053c360c919d3e6aac35755d51e45a5d09621e4f'
+  assert lowering.source_fingerprint(_FINGERPRINTED) == want
+  reindented = textwrap.indent(_FINGERPRINTED.replace('  ', '    '), '    ')
+  commented = _FINGERPRINTED.replace('\n\n', '\n\n  # the update\n\n').replace(
+      'actions == 0:', 'actions == 0:  # north')
+  assert lowering.source_fingerprint(reindented) == want
+  assert lowering.source_fingerprint(commented) == want
+  for edit in [('_north', '_south'), ('== 0', '== 1'), ('otherwise', 'always'),
+               ('del backdrop, things  # unused', 'del backdrop, things, layers')]:
+    assert lowering.source_fingerprint(_FINGERPRINTED.replace(*edit)) != want, edit
+
+
+def test_reference_warehouse_example_loads_and_lowers():
   for level in (0, 1, 2):
-    theirs = lowering.lower(mod.make_game(level))
-    ours = lowering.lower(g_warehouse.make_game(
-        mod.WAREHOUSES_ART[level], mod.WAREHOUSES_WHAT_LIES_BENEATH[level]))
-    _same_lowering(theirs, ours)
+    art, wlb = gc.warehouse_art(gc.load('warehouse_stock_L%d' % level))
+    rt.check_lowering('warehouse_manager_%d' % level,
+                      lowering.lower(g_warehouse.make_game(art, wlb)))
 
 
-@needs_ref
-def test_reference_marauders_example_loads_and_lowers(compat_examples):
-  mod = compat_examples('extraterrestrial_marauders')
-  _same_lowering(lowering.lower(mod.make_game()),
-                 lowering.lower(g_marauders.make_game(levels.marauders_level())))
+def test_reference_marauders_example_loads_and_lowers():
+  rt.check_lowering('extraterrestrial_marauders',
+                    lowering.lower(g_marauders.make_game(levels.marauders_level())))
 
 
-@needs_ref
-def test_reference_example_outside_the_lowered_set_is_refused(compat_examples):
-  # every other example now has a device program; tennis stays out of scope (SURVEY §2)
-  mod = compat_examples('tennnnnnnnnnnnnnnnnnnnnnnnis')
+def test_reference_example_outside_the_lowered_set_is_refused(compat_loader):
+  # a game whose entities carry their own Python update() (tennis, or anything a
+  # user writes) has no device program
+  mod = compat_loader('tennnnnnnnnnnnnnnnnnnnnnnnis', """
+from pycolab import ascii_art
+from pycolab import things
+
+
+class BallSprite(things.Sprite):
+  def update(self, actions, board, layers, backdrop, things, the_plot):
+    self._position = self.Position(self.position.row, (self.position.col + 1) % 5)
+
+
+def make_game():
+  return ascii_art.ascii_art_to_game(['  o  '], ' ', sprites={'o': BallSprite})
+""")
   with pytest.raises(NotLoweredError):
     lowering.lower(mod.make_game())
 
 
-@needs_ref
-def test_reference_better_scrolly_example_loads_and_lowers(compat_examples):
+def test_reference_better_scrolly_example_loads_and_lowers():
   from pycolab_b200.games import better_scrolly_maze as g_better
-  mod = compat_examples('better_scrolly_maze')
   for level in (0, 1, 2):
-    theirs = lowering.lower(mod.make_game(level))
-    ours = lowering.lower(g_better.make_game(mod.MAZES_ART[level]))
-    assert theirs.program == _lib.PROG_BETTER_SCROLLY
-    _same_lowering(theirs, ours)
-  # the example's own croppers are this package's classes
-  views = mod.make_croppers(0)
+    art = [bytes(r).decode('ascii') for r in gc.load('better_stock_L%d' % level)['art']]
+    ours = lowering.lower(g_better.make_game(art))
+    assert ours.program == _lib.PROG_BETTER_SCROLLY
+    rt.check_lowering('better_scrolly_maze_%d' % level, ours)
+  # the example's croppers are this package's classes
+  views = g_better.make_croppers()
   assert [type(v).__name__ for v in views] == ['ScrollingCropper', 'ScrollingCropper',
                                                'FixedCropper']
 
 
-@needs_ref
 @pytest.mark.parametrize('kind', ['four_rooms', 'cliff_walk', 'chain_walk'])
-def test_reference_classics_examples_load_and_lower(compat_examples, kind):
+def test_reference_classics_examples_load_and_lower(kind):
   import importlib
   from oracle import games as ogames
-  mod = compat_examples(os.path.join('classics', kind))
   ours_mod = importlib.import_module('pycolab_b200.games.classics.' + kind)
-  assert list(mod.GAME_ART) == list(ours_mod.GAME_ART)
-  theirs, ours = lowering.lower(mod.make_game()), lowering.lower(ours_mod.make_game())
-  assert theirs.program == _lib.PROG_CLASSICS and theirs.reward_type is float
-  _same_lowering(theirs, ours)
+  ours = lowering.lower(ours_mod.make_game())
+  assert ours.program == _lib.PROG_CLASSICS and ours.reward_type is float
+  rt.check_lowering(kind, ours)
   # ... and the lowered initial state is the oracle's
-  world = ogames.make_classic(kind, list(mod.GAME_ART))
+  world = ogames.make_classic(kind, list(ours_mod.GAME_ART))
   w = world.things['P']
-  assert tuple(theirs.sprites[0, :5]) == (w.row, w.col, w.vrow, w.vcol, 1)
-  np.testing.assert_array_equal(theirs.backdrop[:, :theirs.cols], world.backdrop)
-  assert bool(theirs.confined[0]) == w.confined
+  assert tuple(ours.sprites[0, :5]) == (w.row, w.col, w.vrow, w.vcol, 1)
+  np.testing.assert_array_equal(ours.backdrop[:, :ours.cols], world.backdrop)
+  assert bool(ours.confined[0]) == w.confined
 
 
-@needs_ref
-def test_reference_aperture_example_loads_and_lowers(compat_examples):
+def test_reference_aperture_example_loads_and_lowers():
   from pycolab_b200.games import aperture as ours_mod
-  mod = compat_examples('aperture')
   for level in (0, 1, 2):
-    theirs = lowering.lower(mod.make_game(level))
-    ours = lowering.lower(ours_mod.make_game(mod.LEVELS[level]))
-    assert theirs.program == _lib.PROG_APERTURE
-    assert list(theirs.drapes[0, [_lib.D_AUX0, _lib.D_AUX1]]) == [-1, -1]
-    _same_lowering(theirs, ours)
+    art = [bytes(r).decode('ascii') for r in gc.load('aperture_stock_L%d' % level)['art']]
+    ours = lowering.lower(ours_mod.make_game(art))
+    assert ours.program == _lib.PROG_APERTURE
+    assert list(ours.drapes[0, [_lib.D_AUX0, _lib.D_AUX1]]) == [-1, -1]
+    rt.check_lowering('aperture_%d' % level, ours)
 
 
-@needs_ref
-def test_reference_fluvial_natation_loads_and_lowers(compat_examples):
+def test_reference_fluvial_natation_loads_and_lowers():
   """A Backdrop subclass with update() logic is lowered with its own game only."""
   from pycolab_b200.games import fluvial_natation as ours_mod
-  mod = compat_examples('fluvial_natation')
-  theirs, ours = lowering.lower(mod.make_game()), lowering.lower(ours_mod.make_game())
-  assert theirs.program == _lib.PROG_CLASSICS and theirs.backdrop_role == 'river'
-  assert list(theirs.program_arg[:3]) == [_lib.CLASSIC_FLUVIAL, 1, 4] and theirs.reward_type is int
-  _same_lowering(theirs, ours)
+  from pycolab_b200.games.classics import four_rooms
+  ours = lowering.lower(ours_mod.make_game())
+  assert ours.program == _lib.PROG_CLASSICS and ours.backdrop_role == 'river'
+  assert list(ours.program_arg[:3]) == [_lib.CLASSIC_FLUVIAL, 1, 4] and ours.reward_type is int
+  rt.check_lowering('fluvial_natation', ours)
   # the river under another game's entities is refused, and so is an unknown Backdrop
-  aa = sys.modules['pycolab.ascii_art']
-  four_rooms = compat_examples(os.path.join('classics', 'four_rooms'))
   with pytest.raises(NotLoweredError):
-    lowering.lower(aa.ascii_art_to_game(four_rooms.GAME_ART, ' ',
-                                        sprites={'P': four_rooms.PlayerSprite},
-                                        backdrop=mod.RiverBackdrop))
+    lowering.lower(ascii_art.ascii_art_to_game(four_rooms.GAME_ART, ' ',
+                                               sprites={'P': four_rooms.PlayerSprite},
+                                               backdrop=ours_mod.RiverBackdrop))
 
-  class Odd(mod.RiverBackdrop):
+  class Odd(ours_mod.RiverBackdrop):
     def update(self, *args, **kwargs):
       pass
   with pytest.raises(NotLoweredError):
-    lowering.lower(aa.ascii_art_to_game(mod.GAME_ART, ' ', sprites={'P': mod.PlayerSprite},
-                                        backdrop=Odd))
+    lowering.lower(ascii_art.ascii_art_to_game(ours_mod.GAME_ART, ' ',
+                                               sprites={'P': ours_mod.PlayerSprite},
+                                               backdrop=Odd))
 
 
-@needs_ref
-def test_reference_host_only_unit_tests_pass_against_this_package(compat_examples):
-  """The reference's own unit tests that need no step — ascii_art_test.py and
-  scrolling_test.py::testProtocol (the scrolling-protocol helpers incl. their
-  error messages) — run UNMODIFIED with `pycolab` aliased to this package."""
-  import importlib.util
-  import types
-  import unittest
-  base = os.path.join(refdriver.REFERENCE_ROOT, 'pycolab', 'tests')
-  package = sys.modules.setdefault('pycolab.tests', types.ModuleType('pycolab.tests'))
-
-  def load(name):
-    spec = importlib.util.spec_from_file_location('pycolab.tests.' + name,
-                                                  os.path.join(base, name + '.py'))
-    module = importlib.util.module_from_spec(spec)
-    sys.modules[spec.name] = module
-    setattr(package, name, module)
-    spec.loader.exec_module(module)
-    return module
-  load('test_things')
-  suite = unittest.TestSuite()
-  suite.addTests(unittest.defaultTestLoader.loadTestsFromModule(load('ascii_art_test')))
-  suite.addTest(load('scrolling_test').ScrollingTest('testProtocol'))
-  result = unittest.TextTestRunner(verbosity=0).run(suite)
-  assert result.testsRun == 2 and result.wasSuccessful(), result.failures + result.errors
-
-
-@needs_ref
-def test_reference_test_fixtures_load_and_lower(compat_examples):
-  """The reference's own tests/test_things.py fixtures lower to the general
-  device program, identically to this package's games/fixtures.py."""
-  import sys
-  from pycolab_b200 import compat
+def test_reference_test_fixtures_load_and_lower():
+  """The original's tests/test_things.py fixtures lowered to the general device
+  program exactly as this package's games/fixtures.py does."""
   from pycolab_b200.games import fixtures
-  tt = compat.load_example(os.path.join(refdriver.REFERENCE_ROOT, 'pycolab', 'tests',
-                                        'test_things.py'))
-  g = gc.load('fixture_scrolly_0')
-  kw, cfg = gc.fixture_kwargs(g)
-  aa = sys.modules['pycolab.ascii_art']
-  shape = (len(kw['art']), len(kw['art'][0]))
-  sprites = {ch: aa.Partial(tt.TestMazeWalker, impassable=w.get('impassable', ''),
-                            confined_to_board=w.get('confined', False),
-                            egocentric_scroller=w.get('egocentric', False))
-             for ch, w in kw['walkers'].items()}
-  drapes = {ch: aa.Partial(tt.TestScrolly, board_shape=shape, whole_pattern=s['pattern'],
-                           board_northwest_corner=s['corner'], scroll_margins=s['margins'])
-            for ch, s in kw['scrollys'].items()}
-  theirs = aa.ascii_art_to_game(kw['art'], ' ', sprites, drapes,
-                                update_schedule=kw['update_schedule'],
-                                z_order=kw['z_order'])
-  ours = fixtures.make_game(kw['art'], ' ', kw['walkers'], kw['scrollys'], '',
-                            kw['update_schedule'], kw['z_order'])
-  a, b = lowering.lower(theirs), lowering.lower(ours)
-  assert a.program == _lib.PROG_FIXTURE and a.dynamic_z
-  assert a.drape_kind == [1, 1] and a.egocentric == b.egocentric
-  _same_lowering(a, b)
+  kw, cfg = gc.fixture_kwargs(gc.load('fixture_scrolly_0'))
+  ours = lowering.lower(fixtures.make_game(kw['art'], ' ', kw['walkers'], kw['scrollys'], '',
+                                           kw['update_schedule'], kw['z_order']))
+  assert ours.program == _lib.PROG_FIXTURE and ours.dynamic_z
+  assert ours.drape_kind == [1, 1]
+  rt.check_lowering('test_things_fixture_scrolly_0', ours)
+
+
+def test_reference_host_only_unit_tests_pass_against_this_package():
+  """What the original's host-only unit tests (ascii_art_test.py,
+  scrolling_test.py::testProtocol) check, on this package: malformed art is
+  refused with messages that say what was wrong (and so are malformed entity
+  tables), and the scrolling-protocol helpers register
+  participants per group, grant motions for the next frame only, accept one
+  order per frame and name the offending entity in their errors."""
+  from pycolab_b200 import plot as plot_lib
+  from pycolab_b200.protocols import scrolling
+
+  class Walker(things.Sprite):
+    def update(self, *args, **kwargs):
+      pass
+
+  class Curtain(things.Drape):
+    def update(self, *args, **kwargs):
+      pass
+
+  # ascii_art_to_uint8_nparray: ragged rows, a row that is not a string, rows of
+  # single characters
+  with pytest.raises(ValueError, match='must be a list'):
+    ascii_art.ascii_art_to_uint8_nparray(['ab', 'abc'])
+  with pytest.raises(TypeError, match='must be a list'):
+    ascii_art.ascii_art_to_uint8_nparray(['ab', 12])
+  with pytest.raises(TypeError, match='Did you pass a list of list of single characters'):
+    ascii_art.ascii_art_to_uint8_nparray([['a', 'b'], ['c', 'd']])
+  # ascii_art_to_game: ragged art, a character that is both sprite and drape, a
+  # sprite character appearing twice
+  with pytest.raises(ValueError):
+    ascii_art.ascii_art_to_game(['P ', ' '], ' ', {'P': Walker})
+  with pytest.raises(RuntimeError, match='already being used'):
+    ascii_art.ascii_art_to_game(['P '], ' ', {'P': Walker}, {'P': Curtain})
+  with pytest.raises(ValueError):
+    ascii_art.ascii_art_to_game(['PP'], ' ', {'P': Walker})
+
+  sprite = Walker(things.Sprite.Position(6, 7), things.Sprite.Position(2, 3), 'P')
+  drape = Curtain(np.zeros((6, 7), dtype=bool), 'X')
+  the_plot = plot_lib.Plot()
+  for who in (sprite, drape):
+    scrolling.participate_as_egocentric(who, the_plot, scrolling_group='g')
+  assert scrolling.egocentric_participants(drape, the_plot, scrolling_group='g') == {sprite, drape}
+  assert scrolling.get_order(sprite, the_plot, scrolling_group='g') is None
+  with pytest.raises(scrolling.Error, match="known to belong to scrolling group 'g'"):
+    scrolling.get_order(sprite, the_plot, scrolling_group='h')
+  with pytest.raises(TypeError):
+    scrolling.participate_as_egocentric(object(), the_plot)
+
+  the_plot = plot_lib.Plot()
+  for who in (sprite, drape):
+    scrolling.participate_as_egocentric(who, the_plot)
+  for frame in range(8):                       # the frame counter advances one at a time
+    the_plot.frame = frame
+  scrolling.permit(sprite, the_plot, motions=[(0, 0), (0, -1), (-1, 0)])
+  scrolling.permit(drape, the_plot, motions=[(0, 0), (-1, 0)])
+  assert not any(scrolling.is_possible(drape, the_plot, m) for m in [(0, 0), (-1, 0)])
+  the_plot.frame = 8                           # permits hold for the next frame only
+  assert scrolling.is_possible(sprite, the_plot, (0, 0))
+  assert scrolling.is_possible(sprite, the_plot, (-1, 0))
+  assert not scrolling.is_possible(sprite, the_plot, (0, -1))   # the drape never allowed it
+  with pytest.raises(scrolling.Error, match="impossible scrolling motion"):
+    scrolling.order(drape, the_plot, (0, -1))
+  scrolling.order(drape, the_plot, (-1, 0))
+  assert scrolling.get_order(sprite, the_plot) == (-1, 0)
+  with pytest.raises(scrolling.Error, match="Sprite or Drape handling character 'P'.*second"):
+    scrolling.order(sprite, the_plot, (0, 0))
+  the_plot.frame = 9
+  assert scrolling.get_order(sprite, the_plot) is None
+  assert not scrolling.is_possible(sprite, the_plot, (0, 0))    # permits expired
 
 
 @pytest.mark.parametrize('call', [lambda p: p.add_reward(1), lambda p: p.terminate_episode(),

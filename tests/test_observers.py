@@ -1,10 +1,11 @@
-"""Observation post-processors: oracle vs the reference (CPU), device vs oracle (GPU)."""
+"""Observation post-processors: oracle vs the original (CPU), device vs oracle (GPU)."""
+
+import os
 
 import numpy as np
 import pytest
 
 import golden_cases as gc
-import refdriver
 from oracle import engine_model as em
 
 WAREHOUSE_REPAINT = {c: 'x' for c in '0123456789'}
@@ -19,26 +20,61 @@ def _boards(name, n=6):
   return g['boards'][idx]
 
 
-@pytest.mark.skipif(not refdriver.available(), reason='/root/reference not present')
-def test_oracle_post_processors_match_reference():
-  refdriver._import()
-  from pycolab import rendering as ref
-  for board in _boards('warehouse_stock_L1'):
-    chars = set(' .#_PX0123456789')
-    obs = ref.Observation(board=board, layers={c: board == ord(c) for c in chars})
-    np.testing.assert_array_equal(ref.ObservationCharacterRepainter(WAREHOUSE_REPAINT)(obs).board,
-                                  em.observation_repaint(board, WAREHOUSE_REPAINT))
+def observer_outputs(module, boards):
+  """{name: array} of the post-processors of `module` (the original's
+  `pycolab.rendering` or `oracle_rendering` below) on `boards`."""
+  out = {}
+  chars = set(' .#_PX0123456789')
+  scalar = {c: float(ord(c)) / 2 for c in chars}
+  for i, board in enumerate(boards):
+    obs = module.Observation(board=board, layers={c: board == ord(c) for c in chars})
+    out['repaint_%d' % i] = module.ObservationCharacterRepainter(WAREHOUSE_REPAINT)(obs).board
     for permute in (None, (1, 2, 0), (2, 0, 1)):
-      np.testing.assert_array_equal(
-          ref.ObservationToArray(RGB, dtype=np.uint8, permute=permute)(obs),
-          em.observation_to_array(board, RGB, np.uint8, permute))
-      np.testing.assert_array_equal(
-          ref.ObservationToFeatureArray('P#_0X', permute=permute)(obs),
-          em.observation_to_feature_array(board, 'P#_0X', permute))
-    scalar = {c: float(ord(c)) / 2 for c in chars}
-    np.testing.assert_array_equal(
-        ref.ObservationToArray(scalar, dtype=np.float32, permute=(1, 0))(obs),
-        em.observation_to_array(board, scalar, np.float32, (1, 0)))
+      tag = '%d_%s' % (i, ''.join(map(str, permute or ())))
+      out['rgb_' + tag] = module.ObservationToArray(RGB, dtype=np.uint8, permute=permute)(obs)
+      out['features_' + tag] = module.ObservationToFeatureArray('P#_0X', permute=permute)(obs)
+    out['scalar_%d' % i] = module.ObservationToArray(scalar, dtype=np.float32,
+                                                     permute=(1, 0))(obs)
+  return out
+
+
+class oracle_rendering(object):
+  """The oracle's post-processors behind the original's class names."""
+  class Observation(object):
+    def __init__(self, board, layers):
+      self.board = board
+
+  class ObservationCharacterRepainter(object):
+    def __init__(self, mapping):
+      self.mapping = mapping
+
+    def __call__(self, obs):
+      return oracle_rendering.Observation(em.observation_repaint(obs.board, self.mapping), None)
+
+  class ObservationToArray(object):
+    def __init__(self, value_mapping, dtype, permute):
+      self.args = value_mapping, dtype, permute
+
+    def __call__(self, obs):
+      return em.observation_to_array(obs.board, *self.args)
+
+  class ObservationToFeatureArray(object):
+    def __init__(self, layers, permute):
+      self.args = layers, permute
+
+    def __call__(self, obs):
+      return em.observation_to_feature_array(obs.board, *self.args)
+
+
+def test_oracle_post_processors_match_reference():
+  """Against the original's outputs, stored in tests/golden/reference_observers.npz
+  by tests/golden/make_reference_traces.py."""
+  with np.load(os.path.join(gc.GOLDEN_DIR, 'reference_observers.npz')) as z:
+    want = {k: z[k] for k in z.files}
+  got = observer_outputs(oracle_rendering, _boards('warehouse_stock_L1'))
+  assert sorted(got) == sorted(want)
+  for k in want:
+    np.testing.assert_array_equal(got[k], want[k], err_msg=k)
 
 
 @pytest.mark.gpu

@@ -1,388 +1,128 @@
-"""Live differential tests: oracle restatement vs the REAL reference.
+"""Differential tests: oracle restatement vs the original pycolab.
 
-Run only where /root/reference exists (the build container).  These pin the
-oracle (`oracle/`) to the reference on seeded random action streams for every
-configured game, on stock and generated levels, plus random walks of the
-reference's own MazeWalker/Scrolly test fixtures.
+These pin the oracle (`oracle/`) to the original on seeded random action streams
+for every configured game, on stock and generated levels, plus random walks of
+the original's own MazeWalker/Scrolly test fixtures.  The original's side of
+each comparison is stored in tests/golden/reference_traces.npz (see
+tests/reference_trace.py and tests/golden/make_reference_traces.py).
 """
 
 import os
-import sys
 
 import numpy as np
 import pytest
 
-sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
-
-import refdriver
-from oracle import engine_model as em
+import reference_trace as rt
 from oracle import games
-from pycolab_b200 import levels
 
-pytestmark = pytest.mark.skipif(not refdriver.available(),
-                                reason='/root/reference not present')
-
-
-def _lockstep(make_ref, make_oracle, actions, check_sprites=True):
-  """Step both with auto-reset on game over; compare everything each frame."""
-  ref, ora = make_ref(), make_oracle()
-  r_out, o_out = ref.its_showtime(), ora.its_showtime()
-  episodes = 0
-  for t, a in enumerate(actions):
-    _compare(ref, ora, r_out, o_out, t, check_sprites)
-    if ref.game_over:
-      episodes += 1
-      ref, ora = make_ref(), make_oracle()
-      r_out, o_out = ref.its_showtime(), ora.its_showtime()
-      continue
-    r_out, o_out = ref.play(a), ora.play(a)
-  return episodes
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden',
+                      'reference_traces.npz')
 
 
-def _compare(ref, ora, r_out, o_out, t, check_sprites):
-  np.testing.assert_array_equal(r_out[0].board, o_out[0], err_msg='t=%d' % t)
-  assert refdriver.reward_pair(r_out[1]) == refdriver.reward_pair(o_out[1]), t
-  assert r_out[2] == o_out[2], t
-  assert ref.game_over == ora.game_over, t
-  if check_sprites:
-    for ch, (row, col, vis) in refdriver.snapshot_things(ref).items():
-      w = ora.things[ch]
-      assert (row, col, vis) == (w.row, w.col, bool(w.visible)), (t, ch)
+def _check(key, scenario, *args):
+  """Replay one scenario on the oracle; its trace must be the original's."""
+  with np.load(GOLDEN) as z:
+    want = z[key]
+  trace, facts = scenario(rt.ORACLE, *args)
+  got = trace.result()
+  assert got[-1] == want[-1], '%s: %d records, the original made %d' % (key, got[-1], want[-1])
+  bad = np.flatnonzero(got != want)
+  assert not len(bad), '%s: first difference within records %d..%d' % (
+      key, bad[0] * rt.Trace.EVERY, min((bad[0] + 1) * rt.Trace.EVERY, int(want[-1])))
+  return facts
+
+
+def test_every_scenario_has_a_stored_trace():
+  with np.load(GOLDEN) as z:
+    assert sorted(z.files) == sorted(rt.cases())
 
 
 @pytest.mark.parametrize('level', [0, 1, 2])
 def test_scrolly_maze_stock(level):
-  maze, board, beneath = refdriver.ref_stock_scrolly_art(level)
-  rs = np.random.RandomState(100 + level)
-  actions = rs.randint(0, 5, size=1500).tolist()
-  _lockstep(lambda: refdriver.ref_scrolly_maze(None, None, level=level),
-            lambda: games.make_scrolly_maze(maze, board, '+', beneath), actions)
+  _check('scrolly_stock_%d' % level, rt.scrolly_stock, level)
 
 
 def test_scrolly_maze_stock_with_quit():
-  maze, board, beneath = refdriver.ref_stock_scrolly_art(0)
-  rs = np.random.RandomState(7)
-  actions = rs.randint(0, 6, size=400).tolist()
-  eps = _lockstep(lambda: refdriver.ref_scrolly_maze(None, None, level=0),
-                  lambda: games.make_scrolly_maze(maze, board, '+', beneath),
-                  actions)
-  assert eps > 10
+  assert _check('scrolly_stock_with_quit', rt.scrolly_stock_with_quit)['episodes'] > 10
 
 
 @pytest.mark.parametrize('seed', [0, 1])
 def test_scrolly_maze_generated_64(seed):
-  maze, board, beneath = levels.scrolly_maze_level(seed)
-  rs = np.random.RandomState(seed)
-  # Biased walk so the window actually scrolls a lot.
-  actions = rs.choice([0, 1, 2, 3, 4], size=600,
-                      p=[.3, .15, .3, .15, .1]).tolist()
-  _lockstep(lambda: refdriver.ref_scrolly_maze(maze, board, beneath),
-            lambda: games.make_scrolly_maze(maze, board, '+', beneath), actions)
+  _check('scrolly_generated_64_%d' % seed, rt.scrolly_generated_64, seed)
 
 
 @pytest.mark.parametrize('level', [0, 1, 2])
 def test_warehouse_stock(level):
-  art, wlb = refdriver.ref_stock_warehouse_art(level)
-  rs = np.random.RandomState(200 + level)
-  actions = rs.randint(0, 5, size=1500).tolist()
-  _lockstep(lambda: refdriver.ref_warehouse(None, level=level),
-            lambda: games.make_warehouse(art, wlb), actions)
+  _check('warehouse_stock_%d' % level, rt.warehouse_stock, level)
 
 
 def test_warehouse_generated_80():
-  art = levels.warehouse_level(3)
-  rs = np.random.RandomState(3)
-  actions = rs.randint(0, 4, size=800).tolist()
-  _lockstep(lambda: refdriver.ref_warehouse(art, ' '),
-            lambda: games.make_warehouse(art, ' '), actions)
+  _check('warehouse_generated_80', rt.warehouse_generated_80)
 
 
 def test_marauders_layout_matches_stock():
-  assert levels.marauders_level() == refdriver.ref_stock_marauders_art()
+  from pycolab_b200 import levels
+  art = levels.marauders_level()
+  with np.load(os.path.join(os.path.dirname(GOLDEN), 'marauders_stock_s0.npz')) as z:
+    assert art == [bytes(r).decode('ascii') for r in z['art']]
 
 
 @pytest.mark.parametrize('seed', [0, 1, 2])
 def test_marauders_stock(seed):
-  art = refdriver.ref_stock_marauders_art()
-  rs = np.random.RandomState(300 + seed)
-  actions = rs.randint(0, 4, size=1200).tolist()
-  # The reference draws from the GLOBAL NumPy RNG; the oracle from its own
-  # RandomState.  Seed both identically and never reseed (episodes continue
-  # the same stream, exactly as back-to-back reference episodes would).
-  np.random.seed(seed)
-  rng = np.random.RandomState(seed)
-  eps = _lockstep(lambda: refdriver.ref_marauders(),
-                  lambda: games.make_marauders(art, rng), actions)
-  assert eps >= 1
-
-
-def _random_fixture_case(seed):
-  rs = np.random.RandomState(seed)
-  H, W = int(rs.randint(5, 12)), int(rs.randint(5, 14))
-  art = np.full((H, W), ord(' '), dtype=np.uint8)
-  art[rs.random_sample((H, W)) < 0.25] = ord('#')
-  art[rs.random_sample((H, W)) < 0.1] = ord('%')
-  free = np.argwhere(art == ord(' '))
-  picks = free[rs.permutation(len(free))[:3]]
-  for ch, (r, c) in zip('abc', picks):
-    art[r, c] = ord(ch)
-  walkers = {
-      'a': dict(impassable='#', confined=bool(rs.randint(2))),
-      'b': dict(impassable='#%a', confined=bool(rs.randint(2))),
-      'c': dict(impassable='', confined=False),
-  }
-  schedule = [['a'], ['b', 'c']] if rs.randint(2) else [['a', 'b', 'c']]
-  art = [bytes(r).decode('ascii') for r in art]
-  return art, walkers, schedule, rs
+  # The original draws from the GLOBAL NumPy RNG seeded once, the oracle from its
+  # own RandomState(seed); episodes continue the same stream.
+  assert _check('marauders_stock_%d' % seed, rt.marauders_stock, seed)['episodes'] >= 1
 
 
 @pytest.mark.parametrize('seed', range(8))
 def test_fixture_walkers_random(seed):
-  art, walkers, schedule, rs = _random_fixture_case(seed)
-  T = 300
-  stream = [{ch: int(rs.randint(0, 9)) for ch in 'abc'} for _ in range(T)]
-  ref = refdriver.ref_fixture(art, ' ', walkers, update_schedule=schedule,
-                              z_order='abc')
-  ora = games.make_fixture_world(art, ' ', walkers, update_schedule=schedule,
-                                 z_order='abc')
-  r_out, o_out = ref.its_showtime(), ora.its_showtime()
-  for t, act in enumerate(stream):
-    _compare(ref, ora, r_out, o_out, t, True)
-    r_out = ref.play(refdriver.fixture_actions_to_ref(act))
-    o_out = ora.play(act)
-    for ch in 'abc':
-      want = ref.the_plot['walk_result_' + ch]
-      got = ora.things[ch].last_result
-      assert _result_code(want) == got, (t, ch, want, got)
-      rv = ref.things[ch].virtual_position
-      assert tuple(rv) == ora.things[ch].virtual_position
+  _check('fixture_walkers_%d' % seed, rt.fixture_walkers_random, seed)
 
 
-def _result_code(result):
-  def code(x):
-    return em.EDGE if x == 'edge!' else ord(x)
-  if result is None:
-    return None
-  if isinstance(result, tuple):
-    return tuple(code(x) for x in result)
-  return code(result)
-
-
-@pytest.mark.parametrize('seed,margins', [(0, (2, 3)), (1, None), (2, (1, 1)),
-                                          (3, None), (4, (2, 2)), (5, (1, 2))])
+@pytest.mark.parametrize('seed,margins', rt.FIXTURE_SCROLLY)
 def test_fixture_scrolly_random(seed, margins):
-  rs = np.random.RandomState(1000 + seed)
-  PH, PW, H, W = 17, 23, 8, 11
-  pattern = rs.random_sample((PH, PW)) < 0.2
-  corner = (int(rs.randint(0, PH - H + 1)), int(rs.randint(0, PW - W + 1)))
-  art = np.full((H, W), ord(' '), dtype=np.uint8)
-  art[3, 4] = ord('P')
-  art[5, 7] = ord('q')
-  art = [bytes(r).decode('ascii') for r in art]
-  walkers = {'P': dict(impassable='#', egocentric=True),
-             'q': dict(impassable='#', egocentric=bool(seed % 2))}
-  scrollys = {'#': dict(pattern=pattern, corner=corner, margins=margins)}
-  schedule = [['#'], ['P', 'q']]
-  ref = refdriver.ref_fixture(art, ' ', walkers, scrollys,
-                              update_schedule=schedule, z_order='#Pq')
-  ora = games.make_fixture_world(art, ' ', walkers, scrollys,
-                                 update_schedule=schedule, z_order='#Pq')
-  r_out, o_out = ref.its_showtime(), ora.its_showtime()
-  for t in range(400):
-    _compare(ref, ora, r_out, o_out, t, True)
-    m = int(rs.randint(0, 9))
-    # Everybody in a scrolling group must request the same motion.  The
-    # reference raises when a no-margin Scrolly clips a diagonal order to
-    # (0, 0) (sprites.py:449-454); the oracle must raise at the same frame.
-    try:
-      r_out = ref.play(refdriver.fixture_actions_to_ref(m))
-    except RuntimeError:
-      with pytest.raises(RuntimeError):
-        ora.play(m)
-      assert t > 3
-      return
-    o_out = ora.play(m)
-    np.testing.assert_array_equal(ref.things['#'].curtain,
-                                  ora.things['#'].curtain)
+  raised_at = _check('fixture_scrolly_%d' % seed, rt.fixture_scrolly_random, seed,
+                     margins)['raised_at']
+  assert raised_at is None or raised_at > 3
 
 
 @pytest.mark.parametrize('kind', games.CLASSIC_KINDS)
 @pytest.mark.parametrize('art', ['stock', 'other'])
 def test_classics(kind, art):
-  from pycolab_b200 import levels
-  art = None if art == 'stock' else levels.classic_level(kind)
-  stock = refdriver.ref_classic_art(kind)
-  n_actions = 3 if kind == 'chain_walk' else 6     # includes no-op / unmapped actions
-  actions = np.random.RandomState(len(kind)).randint(0, n_actions, size=2500).tolist()
-  rewards = []
-
-  def make_ref():
-    return refdriver.ref_classic(kind, art)
-  ref, ora = make_ref(), games.make_classic(kind, art or stock)
-  r_out, o_out = ref.its_showtime(), ora.its_showtime()
-  episodes = 0
-  for t, a in enumerate(actions):
-    _compare(ref, ora, r_out, o_out, t, True)
-    assert type(r_out[1]) is type(o_out[1]), (t, r_out[1], o_out[1])   # float rewards
-    rewards.append(r_out[1])
-    if ref.game_over:
-      episodes += 1
-      ref, ora = make_ref(), games.make_classic(kind, art or stock)
-      r_out, o_out = ref.its_showtime(), ora.its_showtime()
-      continue
-    r_out, o_out = ref.play(a), ora.play(a)
-  assert episodes >= 1 and any(r is not None for r in rewards)
-
-
-def aperture_actions(seed, n):
-  """Walks, blaster shots in all directions, idle steps and a rare quit."""
-  rs = np.random.RandomState(seed)
-  return rs.choice(list(range(10)), size=n,
-                   p=[.14, .14, .14, .14, .04, .1, .1, .1, .095, .005]).tolist()
+  facts = _check('classic_%s_%s' % (kind, art), rt.classics, kind, art)
+  assert facts['episodes'] >= 1 and facts['rewards'] > 0
 
 
 @pytest.mark.parametrize('level', [0, 1, 2, 'other'])
 def test_aperture_stock(level):
-  if level == 'other':
-    art = levels.aperture_level()
-    make_ref = lambda: refdriver.ref_aperture(art=art)
-    seed = 43
-  else:
-    art = refdriver.ref_aperture_art(level)
-    make_ref = lambda: refdriver.ref_aperture(level)
-    seed = 40 + level
-  drapes = []
-
-  def check(ref, ora):
-    np.testing.assert_array_equal(ref.things['X'].curtain, ora.things['X'].curtain)
-  ref, ora = make_ref(), games.make_aperture(art)
-  r_out, o_out = ref.its_showtime(), ora.its_showtime()
-  shots = 0
-  for t, a in enumerate(aperture_actions(seed, 3000)):
-    _compare(ref, ora, r_out, o_out, t, True)
-    check(ref, ora)
-    shots += int(ora.things['X'].curtain.sum() > 0)
-    if ref.game_over:
-      ref, ora = make_ref(), games.make_aperture(art)
-      r_out, o_out = ref.its_showtime(), ora.its_showtime()
-      continue
-    r_out, o_out = ref.play(a), ora.play(a)
-  assert shots > 100
+  assert _check('aperture_%s' % level, rt.aperture, level)['shots'] > 100
 
 
 @pytest.mark.parametrize('art', ['stock', 'other'])
 def test_fluvial_natation(art):
-  from pycolab_b200 import levels
-  art = refdriver.ref_fluvial_art() if art == 'stock' else levels.fluvial_level()
-  actions = np.random.RandomState(5).choice([0, 1, 2], size=1500, p=[.2, .6, .2]).tolist()
-  eps = _lockstep(lambda: refdriver.ref_fluvial(art), lambda: games.make_fluvial(art), actions)
-  assert eps > 5
+  assert _check('fluvial_%s' % art, rt.fluvial_natation, art)['episodes'] > 5
 
 
-@pytest.mark.parametrize('pad,margins', [(' ', (None, None)), (None, (2, 3)),
-                                         (' ', (2, 3))])
+@pytest.mark.parametrize('pad,margins', rt.CROPPERS)
 def test_scrolling_cropper(pad, margins):
-  cropping = refdriver._import()['cropping']
-  maze, board, beneath = levels.scrolly_maze_level(5, world_shape=(65, 65),
-                                                   board_shape=(32, 32))
-  ref = refdriver.ref_scrolly_maze(maze, board, beneath)
-  ora = games.make_scrolly_maze(maze, board, '+', beneath)
-  rc = cropping.ScrollingCropper(rows=9, cols=9, to_track=['P'],
-                                 scroll_margins=margins, pad_char=pad)
-  oc = em.ScrollingCrop(9, 9, ['P'], pad_char=pad, scroll_margins=margins)
-  rc.set_engine(ref)
-  oc.set_engine(ora)
-  r_out, o_out = ref.its_showtime(), ora.its_showtime()
-  rs = np.random.RandomState(11)
-  for t in range(300):
-    np.testing.assert_array_equal(rc.crop(r_out[0]).board, oc.crop(o_out[0]))
-    if ref.game_over:
-      break
-    a = int(rs.randint(0, 5))
-    r_out, o_out = ref.play(a), ora.play(a)
+  _check('cropper_%d' % rt.CROPPERS.index((pad, margins)), rt.scrolling_cropper, pad, margins)
 
 
 @pytest.mark.parametrize('seed', range(6))
 def test_ordeal_story_random_walks(seed):
-  """examples/ordeal.py live: the reference's Story vs the chained oracle worlds,
-  every step (current chapter's un-cropped board, summed reward, discount,
-  chapter name, game over), random walks across all three sub-games."""
-  refdriver.ref_storytelling()
-  from pycolab.examples import ordeal as ref_ordeal
-  from test_ordeal import OracleOrdeal
-  rs = np.random.RandomState(500 + seed)
-  story, mine = ref_ordeal.make_game(), OracleOrdeal()
-  story.its_showtime()
-  mine.its_showtime()
-  for t, a in enumerate(rs.choice([0, 1, 2, 3], size=700, p=[.3, .2, .2, .3]).tolist()):
-    if story.game_over:
-      break
-    obs, reward, discount = story.play(a)
-    view, my_reward, my_discount = mine.play(a)
-    assert story.the_plot.this_chapter == mine.chapter, t
-    np.testing.assert_array_equal(obs.board, view, err_msg='t=%d' % t)
-    assert reward == my_reward and discount == my_discount, t
-    assert story.game_over == mine.game_over, t
+  """examples/ordeal.py: the original's Story vs the chained oracle worlds,
+  random walks across all three sub-games."""
+  _check('ordeal_%d' % seed, rt.ordeal_story, seed)
 
 
 def test_apprehend_many_episodes():
-  """examples/apprehend.py live: 200 episodes, the oracle drawing from
-  random.Random(seed) what the reference draws from the seeded global `random`;
-  boards, rewards (value and type), discounts and the float64 registers at 0 ulp."""
-  import random
-  refdriver._import()
-  from pycolab.examples import apprehend as ref_app
-  steps = wins = 0
-  for seed in range(200):
-    random.seed(seed)
-    ref = ref_app.make_game()
-    ora = games.make_apprehend(ref_app.GAME_ART, random.Random(seed))
-    r_out, o_out = ref.its_showtime(), ora.its_showtime()
-    rs = np.random.RandomState(seed)
-    while True:
-      np.testing.assert_array_equal(r_out[0].board, o_out[0])
-      assert r_out[1] == o_out[1] and type(r_out[1]) is type(o_out[1])
-      assert r_out[2] == o_out[2] and ref.game_over == ora.game_over
-      ball = ref.things['b']
-      assert (ball._dx, ball._x_accumulator) == (ora.things['b'].aux['dx'], ora.things['b'].aux['acc'])
-      if ref.game_over:
-        wins += r_out[1] == 1
-        break
-      a = int(rs.randint(0, 3))
-      r_out, o_out = ref.play(a), ora.play(a)
-      steps += 1
-  assert steps > 1500 and wins > 20
+  """examples/apprehend.py: 200 episodes, the oracle drawing from
+  random.Random(seed) what the original draws from the seeded global `random`."""
+  facts = _check('apprehend', rt.apprehend_many_episodes)
+  assert facts['steps'] > 1500 and facts['wins'] > 20
 
 
 @pytest.mark.parametrize('level', ['stock', 'generated'])
 def test_shockwave_many_episodes(level):
-  """examples/shockwave.py live (scipy's distance transform, NumPy's global randint):
-  boards, rewards, discounts and the wave's curtain every step."""
-  refdriver._import()
-  from pycolab.examples import shockwave as ref_shock
-  from pycolab_b200 import levels
-  art = ref_shock.LEVELS[0] if level == 'stock' else levels.shockwave_level(7, 14, 31, 0.5)
-  ref_shock.LEVELS.append(art)
-  steps = ends = 0
-  try:
-    for seed in range(80):
-      np.random.seed(seed)
-      ref = ref_shock.make_game(len(ref_shock.LEVELS) - 1)
-      ora = games.make_shockwave(art, np.random.RandomState(seed))
-      r_out, o_out = ref.its_showtime(), ora.its_showtime()
-      rs = np.random.RandomState(100 + seed)
-      for _ in range(300):
-        np.testing.assert_array_equal(r_out[0].board, o_out[0])
-        np.testing.assert_array_equal(ref.things['@'].curtain, ora.things['@'].curtain)
-        assert r_out[1] == o_out[1] and type(r_out[1]) is type(o_out[1])
-        assert r_out[2] == o_out[2] and ref.game_over == ora.game_over
-        if ref.game_over:
-          ends += 1
-          break
-        a = int(rs.choice([0, 1, 2, 3, 4], p=[.55, .15, .15, .1, .05]))
-        r_out, o_out = ref.play(a), ora.play(a)
-        steps += 1
-  finally:
-    ref_shock.LEVELS.pop()
-  assert steps > 400 and ends > 60
+  facts = _check('shockwave_%s' % level, rt.shockwave_many_episodes, level)
+  assert facts['steps'] > 400 and facts['ends'] > 60

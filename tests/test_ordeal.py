@@ -5,8 +5,9 @@ issue `Plot.change_z_order` on a real game (ordeal.py:182-185).
 Goldens (tests/golden/ordeal_*.npz) are the reference's own Story on BFS-scripted
 walks (sword + victory, no sword + defeat, castle and back, quit) and random walks.
 CPU: the oracle restatement chained like Story does; GPU: this package's Story over
-device-backed Engines and the device cropper; plus, where /root/reference exists,
-the reference's unmodified ordeal.py loaded through `compat`.
+device-backed Engines and the device cropper; plus, where an upstream pycolab
+checkout is named by PYCOLAB_UPSTREAM, its unmodified ordeal.py loaded through
+`compat`.
 """
 
 import os
@@ -15,6 +16,7 @@ import numpy as np
 import pytest
 
 import golden_cases as gc
+import reference_trace as rt
 import refdriver
 import trajectory as tj
 from oracle import engine_model as em
@@ -127,7 +129,7 @@ def test_device_ordeal_z_order_follows_the_battle():
 
 
 @pytest.mark.gpu
-@pytest.mark.skipif(not refdriver.available(), reason='/root/reference not present')
+@pytest.mark.skipif(not refdriver.available(), reason=refdriver.MISSING)
 def test_reference_ordeal_file_runs_on_the_device_through_compat():
   """The reference's own examples/ordeal.py, unmodified: its classes subclass this
   package's prefabs, `lowering` recognises them by source fingerprint, and its
@@ -145,37 +147,13 @@ def test_reference_ordeal_file_runs_on_the_device_through_compat():
     sys.modules.update(saved)
 
 
-@pytest.mark.skipif(not refdriver.available(), reason='/root/reference not present')
 def test_reference_ordeal_chapters_lower_like_the_twins():
-  import sys
-  from pycolab_b200 import compat, lowering
+  """The chapters the original's examples/ordeal.py builds (with its classes and
+  art, ordeal.py:77-93), loaded through `compat`, lowered to what this package's
+  chapters lower to."""
+  from pycolab_b200 import lowering
   from pycolab_b200.games import ordeal
-  saved = {k: v for k, v in sys.modules.items() if k == 'pycolab' or k.startswith('pycolab.')}
-  compat.uninstall()
-  try:
-    mod = compat.load_example(os.path.join(refdriver.REFERENCE_ROOT, 'pycolab', 'examples',
-                                           'ordeal.py'))
-    # the reference builds its chapters inside make_game(): rebuild them here with
-    # ITS classes and art (ordeal.py:77-93)
-    aa = mod.ascii_art
-    theirs = {
-        'castle': aa.ascii_art_to_game(mod.GAME_ART_CASTLE, what_lies_beneath=' ',
-                                       sprites=dict(P=mod.PlayerSprite, D=mod.DragonduckSprite),
-                                       update_schedule=['P', 'D'], z_order=['D', 'P']),
-        'cavern': aa.ascii_art_to_game(mod.GAME_ART_CAVERN, what_lies_beneath=' ',
-                                       sprites=dict(P=mod.PlayerSprite),
-                                       drapes=dict(S=mod.SwordDrape), update_schedule=['P', 'S']),
-        'kansas': aa.ascii_art_to_game(mod.GAME_ART_KANSAS, what_lies_beneath='~',
-                                       sprites=dict(P=mod.PlayerSprite))}
-    mine = {'castle': ordeal.make_castle(), 'cavern': ordeal.make_cavern(),
-            'kansas': ordeal.make_kansas()}
-    for chapter in theirs:
-      a, b = lowering.lower(theirs[chapter]), lowering.lower(mine[chapter])
-      assert a.signature() == b.signature(), chapter
-      for field in ('backdrop', 'sprites', 'drapes', 'plot'):
-        np.testing.assert_array_equal(getattr(a, field), getattr(b, field), err_msg=chapter)
-      for d in a.bits:
-        np.testing.assert_array_equal(a.bits[d], b.bits[d])
-  finally:
-    compat.uninstall()
-    sys.modules.update(saved)
+  mine = {'castle': ordeal.make_castle(), 'cavern': ordeal.make_cavern(),
+          'kansas': ordeal.make_kansas()}
+  for chapter, game in mine.items():
+    rt.check_lowering('ordeal_' + chapter, lowering.lower(game))

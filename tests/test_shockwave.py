@@ -11,7 +11,7 @@ import numpy as np
 import pytest
 
 import golden_cases as gc
-import refdriver
+import reference_trace as rt
 import trajectory as tj
 from oracle import games as ogames
 
@@ -126,22 +126,9 @@ def test_shockwave_lowers_and_validates_on_cpu():
     lowering.lower(shockwave.make_game(levels.shockwave_level(0, 40, 20)))
 
 
-@pytest.mark.skipif(not refdriver.available(), reason='/root/reference not present')
 def test_reference_shockwave_file_lowers_like_the_twin():
-  import sys
-  from pycolab_b200 import compat, lowering
+  """The original's examples/shockwave.py, loaded through `compat`, lowered to
+  what this package's twin lowers to."""
+  from pycolab_b200 import lowering
   from pycolab_b200.games import shockwave
-  saved = {k: v for k, v in sys.modules.items() if k == 'pycolab' or k.startswith('pycolab.')}
-  compat.uninstall()
-  try:
-    mod = compat.load_example(os.path.join(refdriver.REFERENCE_ROOT, 'pycolab', 'examples',
-                                           'shockwave.py'))
-    a, b = lowering.lower(mod.make_game(0)), lowering.lower(shockwave.make_game(0))
-    assert a.signature() == b.signature()
-    for field in ('backdrop', 'sprites', 'drapes', 'plot'):
-      np.testing.assert_array_equal(getattr(a, field), getattr(b, field), err_msg=field)
-    for d in range(3):
-      np.testing.assert_array_equal(a.bits[d], b.bits[d])
-  finally:
-    compat.uninstall()
-    sys.modules.update(saved)
+  rt.check_lowering('shockwave', lowering.lower(shockwave.make_game(0)))
