@@ -12,8 +12,9 @@
 // it.
 //
 // Memory schedule (one warp per env, everything staged through shared memory):
-//   1. records (sprites/drapes/plot, 64 words) -> smem with two coalesced loads;
-//      only the fields this game uses are pulled into registers;
+//   1. records (sprites/drapes/plot, 64 words) -> smem with two coalesced loads (for
+//      the write-back); the fields this game uses go straight to registers with
+//      16-byte loads issued beside them, not through a store to smem and a read back;
 //   2. group 0 ('#' MazeDrape) is pure register arithmetic and fixes BOTH
 //      final window corners (the '@' drape can only obey an order, never issue
 //      one: by the time it runs, the player's permit is already for frame+1);
@@ -31,6 +32,9 @@
 //      segments from smem (prmt with a 256-entry selector table) and streams them
 //      out with uint4 stores; records go back with two coalesced stores.
 // So a step costs ~two dependent DRAM round trips (records, then everything).
+// The 64 x 64 board has its own instantiation of the same body with the shape fixed
+// at compile time (fully unrolled staging / segment / paint loops, constant smem
+// offsets); every other shape runs the instantiation that reads it at run time.
 //
 // Tried and rejected (round 2, A/B on one B200, profiles/r02_step_variants.txt): HALF a
 // warp per env (two envs per warp, every warp primitive on the half's 16-lane mask; the
@@ -201,8 +205,68 @@ __device__ __forceinline__ void scrolly_move_p(Drape& d, const ScrollyCfg& cfg, 
   plot.order_r = orr; plot.order_c = occ; plot.order_frame = plot.frame;
 }
 
+// Phase stamps for tools/step_phases.py: compiled only with -DPCL_STEP_PHASES, nothing
+// in the normal build.  Lane 0 of each warp records %globaltimer and clock64() at
+// kPhases points of the step (entry, after griddepcontrol.wait, records landed, second
+// batch of loads issued, cp.async drained, paint start, paint end) and its %smid.
+#ifdef PCL_STEP_PHASES
+constexpr int kPhases = 7, kPhaseEnvs = 8192, kPhaseWords = 2 * kPhases + 2;
+__device__ unsigned long long g_step_phases[kPhaseEnvs * kPhaseWords];
+__device__ __forceinline__ void phase_stamp(int env, int lane, int i) {
+  if (lane == 0 && env < kPhaseEnvs) {
+    unsigned long long t;
+    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
+    unsigned long long* w = g_step_phases + (size_t)env * kPhaseWords;
+    w[i] = t;
+    w[kPhases + i] = (unsigned long long)clock64();
+    if (i == 0) {
+      unsigned sm;
+      asm volatile("mov.u32 %0, %%smid;" : "=r"(sm));
+      w[2 * kPhases] = sm;
+    }
+  }
+}
+#define PCL_PHASE(i) phase_stamp(env, lane, (i))
+#else
+#define PCL_PHASE(i) ((void)0)
+#endif
+
+// Records: loads of 16 bytes straight from global memory into registers (every lane
+// the same address: one request per warp), issued beside the coalesced copy that
+// goes to shared memory for the write-back, so no field waits for a store to shared
+// memory and a read back.
+__device__ __forceinline__ Sprite load_sprite(const int32_t* r) {
+  const int4 a = *reinterpret_cast<const int4*>(r), b = *reinterpret_cast<const int4*>(r + 4);
+  Sprite s;
+  s.row = a.x; s.col = a.y; s.vrow = a.z; s.vcol = a.w;
+  s.flags = b.x; s.aux0 = b.y; s.aux1 = b.z; s.aux2 = 0;
+  return s;
+}
+__device__ __forceinline__ Drape load_drape(const int32_t* r) {
+  const int4 a = *reinterpret_cast<const int4*>(r), b = *reinterpret_cast<const int4*>(r + 4);
+  Drape d;
+  d.corner_r = a.x; d.corner_c = a.y; d.pre_r = a.z; d.pre_c = a.w;
+  d.last_frame = b.x; d.aux0 = b.y; d.aux1 = b.z; d.aux2 = 0;
+  return d;
+}
+// Plot words 0..8 (frame .. aux0), the ones this game reads.
+__device__ __forceinline__ Plot load_plot(const int32_t* r) {
+  const int4 a = *reinterpret_cast<const int4*>(r), b = *reinterpret_cast<const int4*>(r + 4);
+  Plot pl;
+  pl.frame = a.x; pl.game_over = a.y; pl.error = a.z; pl.episodes = a.w;
+  pl.order_r = b.x; pl.order_c = b.y; pl.order_frame = b.z; pl.ego_mask = b.w;
+  pl.aux0 = r[PCL_P_AUX0];
+  return pl;
+}
+
+// One body for every board shape.  kH / kW > 0 fix the board at compile time (the
+// 64 x 64 board of the generated levels, pitch 64): loop trip counts, shared-memory
+// offsets and the window width are then constants and the general-width code is
+// gone.  kH = kW = 0 takes the shape from the launch parameters (any other board).
+template <int kH, int kW>
 __global__ void __launch_bounds__(kWarpsPerBlock * 32, 7)
 scrolly_maze_step(const StepParams p) {
+  static_assert((kH > 0) == (kW > 0) && kW <= 64 && (kW & 15) == 0, "fixed shape: pitch = W <= 64");
   extern __shared__ __align__(16) uint8_t smem_raw[];
   // Byte-permute selectors for 4 cells at once: index = wall nibble << 4 | coin
   // nibble; selector nibble k picks byte 5 ('#') if wall_k, else byte 4 ('@') if
@@ -217,9 +281,10 @@ scrolly_maze_step(const StepParams p) {
              reinterpret_cast<const uint8_t*>(g_sel.v) + lane * 16);
   pdl_launch_dependents();
   const int env = blockIdx.x * kWarpsPerBlock + warp;
+  PCL_PHASE(0);
   const bool live = env < p.B;
-  const int H = p.H, W = p.W, PWW = p.PWW;
-  const int pitch = p.pitch;
+  const int H = kH ? kH : p.H, W = kW ? kW : p.W, PWW = p.PWW;
+  const int pitch = kW ? kW : p.pitch;
   const int nw = window_words(W);            // staged words per window row (4 for W <= 64)
 
   uint8_t* my = smem_raw + warp * warp_smem_bytes(H, pitch, nw);
@@ -230,6 +295,7 @@ scrolly_maze_step(const StepParams p) {
   // Everything above ran without touching state earlier kernels may have
   // produced (g_sel is a constant); from here on the kernel reads such state.
   pdl_wait_prior_grids();
+  PCL_PHASE(1);
   // An attached cropper reads its corner state at the very end: start that line's trip
   // from DRAM now (a hint, no register held).
   if (p.has_cropper && p.cropper.state && live && lane == 0)
@@ -256,84 +322,60 @@ scrolly_maze_step(const StepParams p) {
     const uint8_t* src = p.st.d_backdrop + lvl * p.st.backdrop_bstride + lane * 16;
     uint8_t* dst = s_bd + lane * 16;
     const int n16 = (H * pitch) >> 4;
-#pragma unroll 4
+#pragma unroll(kH ? kH * kW / 512 : 4)
     for (int i = lane; i < n16; i += 32, src += 512, dst += 512) cp_async16(dst, src);
   }
-  // ---- 1. records -> smem (coalesced) ------------------------------------
+  // ---- 1. records -> registers (the fields this game reads, one lane's walker and
+  // the player, drapes and plot in every lane) and -> smem (coalesced, for the
+  // write-back and the cropper epilogue) ---------------------------------------
+  const int me = lane & 3;                   // ONE walker per lane (P, a, b, c) in group 1
+  Sprite mine = load_sprite(g_sprites + me * PCL_SPRITE_WORDS);
+  Sprite p0 = load_sprite(g_sprites);        // the player: previous render + permits
+  Drape walls = load_drape(g_drapes), coins = load_drape(g_drapes + PCL_DRAPE_WORDS);
+  Plot plot = load_plot(g_plot);
   rec[lane] = g_sprites[lane];
   rec[32 + lane] = lane < 16 ? g_drapes[lane] : g_plot[lane - 16];
-  __syncwarp();
-  const int was_over = rec[48 + PCL_P_GAME_OVER];
   bool restart;                              // engine.py:520-581, 619-624
   bool frozen = false;
   if (p.mode == MODE_RESET) {
     restart = (p.env_mask == nullptr) || (p.env_mask[env] != 0);
     frozen = !restart;
   } else {
-    restart = was_over && p.auto_reset;
-    frozen = was_over && !p.auto_reset;      // reference raises; env stays frozen
+    restart = plot.game_over && p.auto_reset;
+    frozen = plot.game_over && !p.auto_reset;   // reference raises; env stays frozen
   }
   if (frozen) {                              // warp-uniform
     cp_async_wait_all();
     return;
   }
+  PCL_PHASE(2);
   int action;
   if (restart) {
-    const int episodes = rec[48 + PCL_P_EPISODES], error = rec[48 + PCL_P_ERROR];
+    const int episodes = plot.episodes, error = plot.error;
     __syncwarp();
     const int32_t* si = p.st.d_sprites_init + lvl * p.st.sprites_init_bstride;
     const int32_t* di = p.st.d_drapes_init + lvl * p.st.drapes_init_bstride;
     const int32_t* pi = p.st.d_plot_init + lvl * p.st.plot_init_bstride;
     rec[lane] = __ldg(si + lane);
     rec[32 + lane] = lane < 16 ? __ldg(di + lane) : __ldg(pi + lane - 16);
+    mine = load_sprite(si + me * PCL_SPRITE_WORDS);
+    p0 = load_sprite(si);
+    walls = load_drape(di); coins = load_drape(di + PCL_DRAPE_WORDS);
+    plot = load_plot(pi);
+    plot.error = error;
     // Fresh coins: restore the mutable pattern (one Engine per episode).
     const uint32_t* src = p.st.d_pattern_init[1] + lvl * p.st.pattern_init_bstride[1];
     const int n = p.PH * PWW;
     for (int i = lane; i < n; i += 32) coin_pat[i] = __ldg(src + i);
     __syncwarp();
     if (lane == 0) { rec[48 + PCL_P_EPISODES] = episodes + 1; rec[48 + PCL_P_ERROR] = error; }
-    __syncwarp();
     action = PCL_ACTION_NONE;
   } else {
     action = action_early;
   }
-
-  // ---- registers: the drapes / plot / player fields every lane needs, plus ONE
-  // walker per lane (lane & 3: P, a, b, c) for the SIMT part of group 1 ---------
-  const int me = lane & 3;
-  Sprite mine;
-  {
-    const int32_t* r = rec + me * PCL_SPRITE_WORDS;
-    mine.row = r[PCL_S_ROW]; mine.col = r[PCL_S_COL];
-    mine.vrow = r[PCL_S_VROW]; mine.vcol = r[PCL_S_VCOL];
-    mine.flags = r[PCL_S_FLAGS]; mine.aux0 = r[PCL_S_AUX0]; mine.aux1 = r[PCL_S_AUX1];
-    mine.aux2 = 0;
-  }
-  // The player as every lane sees it (previous render + permits).
-  const int p_row = rec[PCL_S_ROW], p_col = rec[PCL_S_COL];
-  const int p_vrow = rec[PCL_S_VROW], p_vcol = rec[PCL_S_VCOL];
-  const bool p_vis = rec[PCL_S_FLAGS] & 1;
-  const int p_permit = rec[PCL_S_AUX0], p_permit_frame = rec[PCL_S_AUX1];
-  Drape walls, coins;
-  {
-    const int32_t* r = rec + 32;
-    walls.corner_r = r[PCL_D_CORNER_R]; walls.corner_c = r[PCL_D_CORNER_C];
-    walls.pre_r = r[PCL_D_PRE_R]; walls.pre_c = r[PCL_D_PRE_C];
-    walls.last_frame = r[PCL_D_LAST_FRAME];
-    r += PCL_DRAPE_WORDS;
-    coins.corner_r = r[PCL_D_CORNER_R]; coins.corner_c = r[PCL_D_CORNER_C];
-    coins.pre_r = r[PCL_D_PRE_R]; coins.pre_c = r[PCL_D_PRE_C];
-    coins.last_frame = r[PCL_D_LAST_FRAME];
-    coins.aux0 = r[PCL_D_AUX0]; coins.aux1 = r[PCL_D_AUX1];
-  }
-  Plot plot;
-  {
-    const int32_t* r = rec + 48;
-    plot.frame = r[PCL_P_FRAME]; plot.error = r[PCL_P_ERROR];
-    plot.order_r = r[PCL_P_ORDER_R]; plot.order_c = r[PCL_P_ORDER_C];
-    plot.order_frame = r[PCL_P_ORDER_FRAME]; plot.ego_mask = r[PCL_P_EGO_MASK];
-    plot.aux0 = r[PCL_P_AUX0];
-  }
+  const int p_row = p0.row, p_col = p0.col, p_vrow = p0.vrow, p_vcol = p0.vcol;
+  const bool p_vis = visible(p0);
+  const int p_permit = p0.aux0, p_permit_frame = p0.aux1;
 
   const ScrollyCfg wcfg = scrolly_cfg(H, W, p.PH, p.PW, p.margin[0][0], p.margin[0][1]);
   const ScrollyCfg ccfg = scrolly_cfg(H, W, p.PH, p.PW, p.margin[1][0], p.margin[1][1]);
@@ -356,6 +398,7 @@ scrolly_maze_step(const StepParams p) {
   const bool narrow = W <= 64;               // the 4-word fast paths (pitch <= 64)
   if (narrow) {
     const int nhalf = H * 2;                 // two 8-byte halves per window row
+#pragma unroll
     for (int i = lane; i < nhalf; i += 32) {
       const int r = i >> 1, k = (i & 1) * 2;
       cp_async8(s_wall + i * 2, wall_pat + (int64_t)(wr + r) * PWW + we + k);
@@ -369,6 +412,7 @@ scrolly_maze_step(const StepParams p) {
       cp_async8(s_coin + i * 2, coin_pat + (int64_t)(cr_pred + r) * PWW + ce + k);
     }
   }
+  PCL_PHASE(3);
   scrolly_touch_prescroll(coins, plot);      // '@' has not moved yet this frame
   // Look-up bits, one pattern ROW per lane: lanes 0..19 = row k of the 5x5 wall
   // patch of walker w (lane = 5 w + k; covers every cell any _check_motion of this
@@ -379,10 +423,11 @@ scrolly_maze_step(const StepParams p) {
   {
     const uint32_t* row = nullptr;
     int c_first = 0, limit = 0;              // first pattern column, words in the row
+    const int w = min(lane / 5, 3), k = lane - w * 5;      // lane w holds walker w
+    const int w_vrow = __shfl_sync(PCL_FULL, mine.vrow, w), w_vcol = __shfl_sync(PCL_FULL, mine.vcol, w);
     if (lane < 20) {
-      const int w = lane / 5, k = lane - w * 5;
-      const int pr = wr + rec[w * PCL_SPRITE_WORDS + PCL_S_VROW] + k - 2;
-      c_first = wc + rec[w * PCL_SPRITE_WORDS + PCL_S_VCOL] - 2;
+      const int pr = wr + w_vrow + k - 2;
+      c_first = wc + w_vcol - 2;
       if ((unsigned)pr < (unsigned)p.PH) { row = wall_pat + (int64_t)pr * PWW; limit = PWW; }
     } else if (lane < 23) {
       const int r = p_vrow + (lane - 20) - 1;
@@ -523,6 +568,7 @@ scrolly_maze_step(const StepParams p) {
 
   // ---- _apply_and_clear_plot (engine.py:761-847); no z-order changes here.
   cp_async_wait_all();
+  PCL_PHASE(4);
   __syncwarp();
   if (lane == 0) {
     int32_t* r = rec + 32;
@@ -575,6 +621,7 @@ scrolly_maze_step(const StepParams p) {
   if (narrow) {
     const uint32_t m_lo = W >= 32 ? 0xffffffffu : (1u << W) - 1u;
     const uint32_t m_hi = W >= 64 ? 0xffffffffu : W > 32 ? (1u << (W - 32)) - 1u : 0u;
+#pragma unroll
     for (int r = lane; r < H; r += 32) {
       const uint4 wv = *reinterpret_cast<const uint4*>(s_wall + r * 4);
       const uint4 cv = *reinterpret_cast<const uint4*>(s_coin + r * 4);
@@ -629,10 +676,12 @@ scrolly_maze_step(const StepParams p) {
   __syncwarp();                              // (also: this warp's s_sel copy has landed, waited above)
   // 5b. The streaming loop: 16 cells per lane per iteration, segment index ==
   // 16-byte index into both the staged tile and the board (pitch = 16 * spr).
+  PCL_PHASE(5);
   const int total = H * spr;
   const unsigned drape_chars = ('#' << 8) | '@';           // bytes 4 and 5 of the permute
   const uint4* src = reinterpret_cast<const uint4*>(s_bd);
   uint4* dst = reinterpret_cast<uint4*>(p.out.d_board + (int64_t)env * H * pitch);
+#pragma unroll
   for (int seg = lane; seg < total; seg += 32) {
     uint4 px = src[seg];
     const uint32_t bits = s_seg[seg];
@@ -642,6 +691,7 @@ scrolly_maze_step(const StepParams p) {
     px.w = prmt(px.w, drape_chars, s_sel[((bits >> 24) & 0xf0u) | ((bits >> 12) & 0xfu)]);
     dst[seg] = px;
   }
+  PCL_PHASE(6);
   // ---- 6. an attached cropper (pcl_attach_cropper): the egocentric view of the board
   // this warp has just stored, without a second kernel (ScrollingCropper.crop,
   // cropping.py:393-426).
@@ -653,14 +703,27 @@ scrolly_maze_step(const StepParams p) {
 
 }  // namespace
 
+#ifdef PCL_STEP_PHASES
+// Copies the stamps of the last launch: kPhaseEnvs rows of kPhaseWords u64 (globaltimer
+// x kPhases, clock64 x kPhases, smid, unused).  Exists only in the stamped build.
+extern "C" int pcl_step_phases_read(void* host, size_t bytes) {
+  if (bytes > sizeof(g_step_phases)) bytes = sizeof(g_step_phases);
+  return (int)cudaMemcpyFromSymbol(host, g_step_phases, bytes);
+}
+#endif
+
 cudaError_t launch_scrolly_maze(const StepParams& p, cudaStream_t s) {
   if (p.PWW & 1) return cudaErrorInvalidValue;   // window rows are staged in 8-byte halves
   const int blocks = (p.B + kWarpsPerBlock - 1) / kWarpsPerBlock;
   const size_t smem = warp_smem_bytes(p.H, p.pitch, window_words(p.W)) * kWarpsPerBlock;
   if (smem > 227 * 1024) return cudaErrorInvalidValue;         // board too large for one CTA
+  // The 64 x 64 board (pitch 64) has its own instantiation; every other shape runs
+  // the one that reads the shape from `p`.
+  void (*kernel)(const StepParams) = (p.H == 64 && p.W == 64 && p.pitch == 64)
+                                         ? scrolly_maze_step<64, 64> : scrolly_maze_step<0, 0>;
   if (smem > 48 * 1024) {   // opt in per launch: the attribute is per device, handles are not
-    cudaError_t e = cudaFuncSetAttribute(scrolly_maze_step,
-                                         cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                         (int)smem);
     if (e != cudaSuccess) return e;
   }
   // Programmatic dependent launch: this kernel may start (prologue only) before
@@ -676,7 +739,7 @@ cudaError_t launch_scrolly_maze(const StepParams& p, cudaStream_t s) {
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
-  return cudaLaunchKernelEx(&cfg, scrolly_maze_step, p);
+  return cudaLaunchKernelEx(&cfg, kernel, p);
 }
 
 }  // namespace pcl

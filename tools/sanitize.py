@@ -4,7 +4,7 @@
     compute-sanitizer --tool memcheck  python tools/sanitize.py
     compute-sanitizer --tool racecheck python tools/sanitize.py
 
-Small shapes (ragged last blocks, boards that are not multiples of 16 columns,
+Small batches (ragged last blocks, the 64 x 64 board, boards that are not multiples of 16 columns,
 auto-resets inside the run) so that out-of-bounds accesses and shared-memory
 hazards would show.  Prints one line per kernel family; the sanitizer's summary
 goes to profiles/ (SURVEY.md §5).
@@ -62,6 +62,13 @@ def main():
   print('ok crop / layers / export / observe / handoff kernels')
   wide = levels.scrolly_maze_level(9, world_shape=(41, 161), board_shape=(12, 100))
   run('scrolly_maze_step W=100', [scrolly_maze.make_game(*wide)], 5, 5)
+  big = [levels.scrolly_maze_level(11 + i) for i in range(2)]        # the fixed-shape instantiation
+  eng = run('scrolly_maze_step 64x64', [scrolly_maze.make_game(*a) for a in big], 7, 6)
+  eng.attach_cropper(spec)
+  for _ in range(6):
+    eng.play(torch.from_numpy(rs.randint(0, 6, size=7).astype(np.int32)).cuda())
+  torch.cuda.synchronize()
+  print('ok scrolly_maze_step 64x64 + attached cropper')
   run('warehouse_step', [warehouse_manager.make_game(
       levels.warehouse_level(3, shape=(14, 21), num_boxes=4, num_goals=5))], 9, 6)
   run('marauders_step', [extraterrestrial_marauders.make_game(levels.marauders_level())], 6, 4,
