@@ -85,6 +85,17 @@ typedef enum pcl_program {
                                 d_bits[0], record AUX0 = impact cell index, AUX1 = steps since impact), ' '
                                 and '^' (static, d_bits_init[1..2]); program_arg[0] = ring width; d_rng =
                                 NumPy RandomState words (np.random.randint picks the impact cell) */
+  PCL_PROG_BOX_WORLD = 12,   /* examples/research/box_world/box_world.py:127-271: one MazeWalker (the
+                                player, '.') and up to 41 key / lock / gem drapes, held together as
+                                ONE byte plane in d_bits[0] / d_bits_init[0] (u8 [*, rows, pitch],
+                                bits_words = pitch / 4): byte = the drape character covering the
+                                cell, 0 = none, bit 7 set on distractor lock cells; cell (0, 0) =
+                                the key held.  n_drapes = 0.  Sprite AUX0 = move actions taken,
+                                AUX1 = max_num_steps.  Boards up to 32 x 32 with '#' all round.
+                                Level rotation: program_arg[1] = stride (0 = off), program_arg[2]
+                                = number of levels; an AUTO-reset sets d_level[env] = (d_level[env]
+                                + stride) % levels before restoring the templates (pcl_reset
+                                restarts the same level) */
   PCL_PROG_ORDEAL = 8        /* examples/ordeal.py:74-266: program_arg[0] = PCL_ORDEAL_* chapter;
                                 plot words AUX0 has_sword, AUX1 last_position (row << 16 | col,
                                 -1 unset), AUX2 next_chapter chosen on the device, AUX3 prior chapter */
@@ -207,8 +218,9 @@ typedef struct pcl_state {
    * static data.  When d_level (i32 [B]) is non-NULL, every array the step never
    * writes — d_backdrop, read-only patterns, every *_init template — is indexed
    * by d_level[env] instead of env (the *_bstride is then the per-LEVEL stride);
-   * mutable arrays stay env-indexed.  NULL = env-indexed (or bstride 0). */
-  const int32_t* d_level;
+   * mutable arrays stay env-indexed.  NULL = env-indexed (or bstride 0).  The
+   * library writes it only for PCL_PROG_BOX_WORLD with level rotation on. */
+  int32_t* d_level;
 } pcl_state;
 
 /* Per-step outputs = the (observation, reward, discount) triple of

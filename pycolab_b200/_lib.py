@@ -38,7 +38,7 @@ ENV_ERR_BAD_Z = 0x10
 
 PROG_NONE, PROG_SCROLLY_MAZE, PROG_WAREHOUSE, PROG_MARAUDERS, PROG_FIXTURE = 0, 1, 2, 3, 4
 PROG_BETTER_SCROLLY, PROG_CLASSICS, PROG_APERTURE, PROG_ORDEAL, PROG_HELLO = 5, 6, 7, 8, 9
-PROG_APPREHEND, PROG_SHOCKWAVE = 10, 11
+PROG_APPREHEND, PROG_SHOCKWAVE, PROG_BOX_WORLD = 10, 11, 12
 ORDEAL_NEXT_UNSET, ORDEAL_NEXT_NONE, ORDEAL_CASTLE, ORDEAL_CAVERN, ORDEAL_KANSAS = -1, 0, 1, 2, 3
 CLASSIC_FOUR_ROOMS, CLASSIC_CLIFF_WALK, CLASSIC_CHAIN_WALK, CLASSIC_FLUVIAL = 0, 1, 2, 3
 

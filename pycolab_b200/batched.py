@@ -42,7 +42,8 @@ class StepResult(object):
 class BatchedEngine(object):
 
   def __init__(self, games, batch=None, device=0, auto_reset=True, rng_seed=0,
-               env_offset=0, rng_states=None, share_levels=True):
+               env_offset=0, rng_states=None, share_levels=True, cycle_levels=False,
+               level_stride=None):
     """games: list of lowered games (`lowering.LoweredGame`) or set-up `Engine`s.
     Env e uses games[e % len(games)]; with a single game the static level data
     (backdrop, immutable patterns, reset templates) is shared by all envs.
@@ -52,11 +53,14 @@ class BatchedEngine(object):
     (False: bind no RNG, for programs that can take their draws from the templates)
     MT19937 states (624 key words + position) instead of seeds.
     share_levels=False stores the static level data once PER ENV instead of once
-    per level (the reference's layout: every Engine owns its backdrop)."""
+    per level (the reference's layout: every Engine owns its backdrop).
+    cycle_levels=True (Box-World only, more than one level, shared levels): the pool
+    is walked instead of pinned: env e starts on level (env_offset + e) % n and every
+    auto-reset moves it on by `level_stride` levels (default: the batch), so envs
+    e, e + B, e + 2B, ... cover the whole pool.  A masked reset() restarts the same
+    level."""
     torch = _torch()
     self._lib = _lib.load()
-    if not torch.cuda.is_available():
-      raise _lib.PclLibraryError('CUDA device required: pycolab_b200 has no CPU path')
     games = [g if isinstance(g, lowering.LoweredGame) else lowering.lower(g)
              for g in (games if isinstance(games, (list, tuple)) else [games])]
     sig = games[0].signature()
@@ -65,6 +69,21 @@ class BatchedEngine(object):
         raise ValueError('all games of one BatchedEngine must share one structure')
     self.game = g0 = games[0]
     self.batch = B = int(batch if batch is not None else len(games))
+    if cycle_levels:
+      if g0.program != _lib.PROG_BOX_WORLD:
+        raise ValueError('cycle_levels is supported for the box_world program only')
+      if len(games) < 2:
+        raise ValueError('cycle_levels needs more than one level')
+      if not share_levels:
+        raise ValueError('cycle_levels needs share_levels=True (envs change level)')
+      level_stride = B if level_stride is None else int(level_stride)
+      if level_stride < 1:
+        raise ValueError('level_stride must be positive')
+    elif level_stride is not None:
+      raise ValueError('level_stride is meaningful with cycle_levels only')
+    self.cycle_levels = bool(cycle_levels)
+    if not torch.cuda.is_available():
+      raise _lib.PclLibraryError('CUDA device required: pycolab_b200 has no CPU path')
     self.device = torch.device('cuda', device)
     self.auto_reset = bool(auto_reset)
     self.rows, self.cols, self.pitch = g0.rows, g0.cols, g0.pitch
@@ -96,7 +115,9 @@ class BatchedEngine(object):
     st = _lib.State()
     self.level = None           # i32 [B]: which level each env plays
     if not shared:
-      self.level = (torch.arange(B, dtype=torch.int32, device=dev) % n).contiguous()
+      first = env_offset if cycle_levels else 0
+      self.level = ((torch.arange(B, dtype=torch.int64, device=dev) + first) % n).to(
+          torch.int32).contiguous()
       st.d_level = self.level.data_ptr()
     self.backdrop = tiled([g.backdrop for g in games], np.uint8)
     st.d_backdrop, st.backdrop_bstride = self.backdrop.data_ptr(), bstride(self.backdrop)
@@ -189,6 +210,8 @@ class BatchedEngine(object):
     self._attached = None       # attach_cropper: (spec, state, out, runs inside the step kernel)
 
     self._spec = g0.make_spec(self.auto_reset)
+    if cycle_levels:
+      self._spec.program_arg[1], self._spec.program_arg[2] = level_stride, n
     handle = C.c_void_p()
     _lib.check(self._lib.pcl_create(C.byref(self._spec), B, self.device.index,
                                     C.byref(handle)), 'pcl_create')
@@ -334,7 +357,17 @@ class BatchedEngine(object):
   # ------------------------------------------------------------- accessors
   def curtain(self, char):
     """Drape.curtain of every env as bool [B, rows, cols] (things.py:213-217)."""
+    if self.game.program == _lib.PROG_BOX_WORLD:
+      # every key, lock and gem lives in the cell plane: byte = character | distractor bit
+      return (self.plane()[:, :, :self.cols] & 0x7f) == ord(char)
     return self._curtain_bytes(self.drape_chars.index(char))[:, :, :self.cols].bool()
+
+  def plane(self):
+    """Box-World cell plane of every env, u8 [B, rows, pitch] (a view of the live
+    state, see pcl.h PCL_PROG_BOX_WORLD)."""
+    if self.game.program != _lib.PROG_BOX_WORLD:
+      raise ValueError('only the box_world program keeps a cell plane')
+    return self.bits[0].view(_torch().uint8)
 
   def _curtain_bytes(self, d):
     """Curtain of drape `d` as u8 [B, rows, pitch] (the pcl_export_curtain layout)."""

@@ -251,6 +251,21 @@ int validate(const pcl_spec& s) {
       if (want_d && s.bits_words < (s.cols + 31) / 32 + 1) return PCL_ERR_INVALID;
       return PCL_OK;
     }
+    case PCL_PROG_BOX_WORLD: {
+      // The player alone is an entity of the spec; the drapes live in the cell plane.
+      if (s.n_sprites != 1 || s.n_drapes != 0) return PCL_ERR_UNSUPPORTED;
+      const int lens[1] = {1};
+      if (!groups_are(s, (const char*)s.sprite_char, lens, 1) || s.z_order[0] != s.sprite_char[0])
+        return PCL_ERR_UNSUPPORTED;
+      if (!s.sprite_confined[0] || s.sprite_egocentric[0] || !set_is(s.impassable[0], "#"))
+        return PCL_ERR_UNSUPPORTED;
+      // a plane of at most 64 16-byte row segments: two per lane of the env's warp
+      if (s.rows > 32 || s.cols > 32 || s.pitch > 32) return PCL_ERR_UNSUPPORTED;
+      if (s.rows < 3 || s.cols < 3 || s.bits_words * 4 != s.pitch) return PCL_ERR_INVALID;
+      const int stride = s.program_arg[1], levels = s.program_arg[2];
+      if (stride < 0 || levels < 0 || (stride > 0 && levels < 1)) return PCL_ERR_INVALID;
+      return PCL_OK;
+    }
     case PCL_PROG_FIXTURE: {
       // Any MazeWalker / Scrolly / plain-drape mix; entities and z-order must
       // be consistent permutations of each other.
@@ -323,6 +338,7 @@ int launch(pcl_handle* h, const StepParams& p, cudaStream_t stream) {
     case PCL_PROG_HELLO: e = pcl::launch_hello(p, stream); break;
     case PCL_PROG_APPREHEND: e = pcl::launch_apprehend(p, stream); break;
     case PCL_PROG_SHOCKWAVE: e = pcl::launch_shockwave(p, stream); break;
+    case PCL_PROG_BOX_WORLD: e = pcl::launch_box_world(p, stream); break;
     default: return PCL_ERR_UNSUPPORTED;
   }
   if (e != cudaSuccess) return cuda_failed(h, e, "step kernel launch");
@@ -437,6 +453,10 @@ int pcl_bind_state(pcl_handle* h, const pcl_state* st) {
   }
   if (h->spec.program == PCL_PROG_BETTER_SCROLLY) {
     if (!st->d_bits[0] || !st->d_bits_init[0] || st->bits_bstride[0] == 0) return PCL_ERR_INVALID;
+  }
+  if (h->spec.program == PCL_PROG_BOX_WORLD) {
+    if (!st->d_bits[0] || !st->d_bits_init[0] || st->bits_bstride[0] == 0) return PCL_ERR_INVALID;
+    if (h->spec.program_arg[1] > 0 && !st->d_level) return PCL_ERR_INVALID;   // rotation writes it
   }
   if (h->spec.n_scroll_groups > 1 && (!st->d_groups || !st->d_groups_init)) return PCL_ERR_INVALID;
   if (h->spec.program == PCL_PROG_FIXTURE) {
@@ -673,6 +693,7 @@ int pcl_layers(pcl_handle* h, const uint8_t* chars, int32_t n_chars, uint8_t* d_
     return PCL_ERR_INVALID;
   if (!h->bound) return PCL_ERR_UNBOUND;
   const pcl_spec& sp = h->spec;
+  if (sp.program == PCL_PROG_BOX_WORLD) return PCL_ERR_UNSUPPORTED;   // drapes held in the cell plane
   pcl::LayersParams p;
   memset(&p, 0, sizeof(p));
   p.B = h->batch; p.H = sp.rows; p.W = sp.cols; p.pitch = sp.pitch;

@@ -62,6 +62,7 @@ cudaError_t launch_ordeal(const StepParams& p, cudaStream_t s);
 cudaError_t launch_hello(const StepParams& p, cudaStream_t s);
 cudaError_t launch_apprehend(const StepParams& p, cudaStream_t s);
 cudaError_t launch_shockwave(const StepParams& p, cudaStream_t s);
+cudaError_t launch_box_world(const StepParams& p, cudaStream_t s);
 
 struct RenderParams {
   int B, H, W, pitch, S, D;

@@ -29,10 +29,16 @@ def make_shard_engine(games, global_batch, rank, world, device, **kwargs):
   """`BatchedEngine` for this rank's block of a `global_batch`-env job.
 
   games[i] is the level of GLOBAL env i (mod len(games)): the local list is
-  rotated so that local env e maps to global env first + e."""
+  rotated so that local env e maps to global env first + e.  With
+  cycle_levels=True every shard keeps the whole pool and steps through it by the
+  GLOBAL batch, so the shards together walk it as one engine would."""
   from pycolab_b200 import batched
   first, count = shard_range(global_batch, rank, world)
   n = len(games)
+  if kwargs.get('cycle_levels'):
+    kwargs.setdefault('level_stride', global_batch)
+    return batched.BatchedEngine(list(games), batch=count, device=device, env_offset=first,
+                                 **kwargs)
   local = [games[(first + i) % n] for i in range(min(n, count))] if n > 1 else games
   return batched.BatchedEngine(local, batch=count, device=device, env_offset=first,
                                **kwargs)

@@ -242,6 +242,13 @@ class Engine(object):
       ent._visible = bool(rec[_lib.S_FLAGS] & 1)
       if isinstance(ent, prefab_sprites.MazeWalker):
         ent._virtual_row, ent._virtual_col = int(rec[_lib.S_VROW]), int(rec[_lib.S_VCOL])
+    if b.game.program == _lib.PROG_BOX_WORLD:
+      # the keys, locks and gem live in one cell plane; the player counts its moves
+      chars = b.plane()[0, :, :self._cols].cpu().numpy() & 0x7f
+      for ch, ent in self._sprites_and_drapes.items():
+        if isinstance(ent, things.Drape):
+          np.copyto(ent.curtain, chars == ord(ch))
+      self._sprites_and_drapes[b.sprite_chars[0]]._step_counter = int(sprites[0, _lib.S_AUX0])
     for i, ch in enumerate(b.drape_chars):
       ent, rec = self._sprites_and_drapes[ch], drapes[i]
       if isinstance(ent, prefab_drapes.Scrolly):

@@ -60,6 +60,10 @@ LOWERED_CLASSES = {
     ('ordeal', 'PlayerSprite'): 'ordeal.player',
     ('ordeal', 'DragonduckSprite'): 'ordeal.dragonduck',
     ('ordeal', 'SwordDrape'): 'ordeal.sword',
+    ('box_world', 'PlayerSprite'): 'box_world.player',
+    ('box_world', 'GemDrape'): 'box_world.gem',
+    ('box_world', 'KeyDrape'): 'box_world.key',
+    ('box_world', 'LockDrape'): 'box_world.lock',
     # General entities: the reference's test fixtures and this package's twins.
     ('test_things', 'TestMazeWalker'): 'fixture.walker',
     ('test_things', 'TestScrolly'): 'fixture.scrolly',
@@ -68,6 +72,11 @@ LOWERED_CLASSES = {
     ('fixtures', 'FixtureScrolly'): 'fixture.scrolly',
     ('fixtures', 'FixtureDrape'): 'fixture.drape',
 }
+
+# Base classes that hold part of a lowered class's rules without being lowered
+# themselves: a class from outside this package that derives from one must carry the
+# original's source for it too (BoxThing.is_locked_at / where_player_over_me).
+FINGERPRINTED_BASES = {('box_world', 'BoxThing')}
 
 # Backdrop subclasses whose update() has a device counterpart.
 LOWERED_BACKDROPS = {
@@ -612,6 +621,147 @@ def _lower_shockwave(engine, roles):
   return game
 
 
+# What the box-world program restates of box_world.py's module constants: an edited
+# copy could change them without touching a class body.
+_BOX_WORLD_CONSTANTS = {
+    'GEM': '*', 'PLAYER': '.', 'BORDER': '#',
+    'KEYS': list('abcdefghijklmnopqrst'), 'LOCKS': list('ABCDEFGHIJKLMNOPQRST'),
+    'REWARD_GOAL': 10., 'REWARD_STEP': 0., 'REWARD_OPEN_CORRECT': 1.,
+    'REWARD_OPEN_WRONG': -1.,
+    'ACTION_MAP': {0: (-1, 0), 1: (1, 0), 2: (0, -1), 3: (0, 1)},
+}
+
+
+def _same_constant(got, want):
+  if isinstance(want, dict):
+    return (isinstance(got, dict) and set(got) == set(want) and
+            all(tuple(got[k]) == want[k] for k in want))
+  if isinstance(want, float):
+    return isinstance(got, (int, float)) and not isinstance(got, bool) and got == want
+  return type(got) is type(want) and got == want
+
+
+def _check_box_world_module(klass):
+  """The module that defines `klass` (whose methods read its globals) must hold the
+  original's constants."""
+  import sys
+  module = sys.modules.get(klass.__module__)
+  for name, want in _BOX_WORLD_CONSTANTS.items():
+    if not _same_constant(getattr(module, name, None), want):
+      raise NotLoweredError('box_world program: {}.{} = {!r} differs from the original\'s '
+                            '{!r}'.format(klass.__module__, name,
+                                          getattr(module, name, None), want))
+
+
+def _box_world_classes(entity):
+  """Classes along the MRO of a box-world entity whose code the device restates: the
+  lowered class and, for drapes, BoxThing.  Classes from outside this package must
+  carry the original's source; subclasses may not override the rules' helpers."""
+  cls = type(entity)
+  out = []
+  for klass in cls.__mro__:
+    key = (klass.__module__.rsplit('.', 1)[-1], klass.__name__)
+    if key in LOWERED_CLASSES or key in FINGERPRINTED_BASES:
+      if key in FINGERPRINTED_BASES and not _is_known_implementation(klass, key):
+        raise NotLoweredError(
+            'class {}.{} is named like {}.{} but its source differs from the original\'s; '
+            'edited copies are not replaced by the stock kernel'.format(
+                klass.__module__, klass.__name__, *key))
+      out.append(klass)
+  for klass in out:
+    for name in ('_in_direction', 'is_locked_at', 'where_player_over_me'):
+      if hasattr(klass, name) and getattr(cls, name) is not getattr(klass, name):
+        raise NotLoweredError('{} overrides {}() of {}.{}'.format(
+            cls.__name__, name, klass.__module__, klass.__name__))
+  if (not isinstance(entity, prefab_sprites.MazeWalker) and
+      not any(k.__name__ == 'BoxThing' for k in out)):
+    raise NotLoweredError('box_world drape {!r} does not derive from BoxThing'.format(
+        entity.character))
+  return out
+
+
+def _lower_box_world(engine, roles):
+  """examples/research/box_world/box_world.py:127-445: the player '.' and any number
+  of key, lock and gem drapes, all in ONE update group [player] + sorted(drapes) and
+  drawn in sorted(drapes) + [player].  The drapes never overlap, so they travel as one
+  byte plane (pcl.h PCL_PROG_BOX_WORLD): the spec names the player alone, and every
+  level of any drape set shares one signature."""
+  th = engine.things
+  kinds = {'box_world.player': '.', 'box_world.gem': '*'}
+  for ch, role in roles.items():
+    if role in ('box_world.key', 'box_world.lock'):
+      upper = role == 'box_world.lock'
+      ok = len(ch) == 1 and ch.isascii() and ch.isalpha() and ch.isupper() == upper and \
+          ord(ch.lower()) - ord('a') < 20
+    else:
+      ok = ch == kinds[role]
+    if not ok:
+      raise NotLoweredError('box_world program: character {!r} cannot be a {}'.format(
+          ch, role.split('.')[1]))
+  if list(roles.values()).count('box_world.player') != 1:
+    raise NotLoweredError('box_world program needs exactly one PlayerSprite')
+  for ent in th.values():
+    for klass in _box_world_classes(ent):
+      _check_box_world_module(klass)
+  game = LoweredGame()
+  _common(engine, game, _lib.PROG_BOX_WORLD)
+  drapes = sorted(ch for ch in roles if ch != '.')
+  if game.groups != ['.' + ''.join(drapes)]:
+    raise NotLoweredError('box_world program needs one update group [player] + '
+                          'sorted(drapes) (got {})'.format(game.groups))
+  if game.z_order != ''.join(drapes) + '.':
+    raise NotLoweredError('box_world program needs z_order sorted(drapes) + [player] '
+                          '(got {!r})'.format(game.z_order))
+  if engine.rows > 32 or engine.cols > 32:
+    raise NotLoweredError('box_world program: boards up to 32 x 32 (grid_size <= 30)')
+  room = np.full((engine.rows, engine.cols), ord(' '), dtype=np.uint8)
+  room[[0, -1], :] = room[:, [0, -1]] = ord('#')
+  if not np.array_equal(engine.backdrop.curtain, room):
+    raise NotLoweredError("box_world program: the backdrop must be a room of ' ' walled "
+                          "by '#'")
+  pl = th['.']
+  impassable, confined, egocentric = _walker_meta(pl)
+  if impassable != char_set_mask('#') or not confined or egocentric:
+    raise NotLoweredError("box_world program: the player is confined and stopped by '#' "
+                          "alone")
+  if not pl.visible or tuple(pl.virtual_position) != tuple(pl.position):
+    raise NotLoweredError('box_world program: the player starts visible on the board')
+  game.pitch = round_up(engine.cols, 16)
+  game.bits_words = game.pitch // 4
+  plane = np.zeros((engine.rows, game.pitch), dtype=np.uint8)
+  for ch in drapes:
+    curtain = th[ch].curtain
+    if np.any(plane[:, :engine.cols][curtain]):
+      raise NotLoweredError('box_world program: drapes overlap at set-up')
+    plane[:, :engine.cols][curtain] = ord(ch)
+    if ch in 'ABCDEFGHIJKLMNOPQRST' and th[ch].key_that_opens != ch.lower():
+      raise NotLoweredError('box_world lock {!r} opens with {!r}'.format(
+          ch, th[ch].key_that_opens))
+  if np.any(plane[[0, -1], :]) or np.any(plane[:, [0, engine.cols - 1]]):
+    raise NotLoweredError('box_world program: no drape on the wall at set-up')
+  for x, y in pl.distractors:
+    x, y = int(x), int(y)
+    if 0 <= y < engine.rows and 0 <= x < engine.cols and chr(plane[y, x]).isupper():
+      plane[y, x] |= 0x80               # only a lock cell's membership is ever asked
+  steps, limit = pl._step_counter, pl._max_num_steps
+  if not all(isinstance(v, (int, np.integer)) for v in (steps, limit)):
+    raise NotLoweredError('box_world program: integer step counts only')
+  game.sprite_chars = '.'
+  game.impassable = [char_set_mask('#')]
+  game.confined = [True]
+  game.egocentric = [False]
+  game.sprites = np.array([_sprite_record(pl, aux0=steps, aux1=limit)], dtype=np.int32)
+  game.z_order = '.'
+  game.groups = ['.']
+  game.drape_chars = ''
+  game.margins = []
+  game.drapes = np.zeros((0, _lib.DRAPE_WORDS), dtype=np.int32)
+  game.bits = {0: plane}
+  game.plot = np.array(_plot_record(), dtype=np.int32)
+  game.reward_type = float                      # box_world.py pays 0.0 / 1.0 / -1.0 / 10.0
+  return game
+
+
 def _update_order(engine):
   return [e.character for _, ents in sorted(engine._update_groups.items()) for e in ents]
 
@@ -783,7 +933,7 @@ def lower(engine):
               'classics': _lower_classics, 'better': _lower_better_scrolly,
               'aperture': _lower_aperture, 'ordeal': _lower_ordeal,
               'hello': _lower_hello, 'apprehend': _lower_apprehend,
-              'shockwave': _lower_shockwave}
+              'shockwave': _lower_shockwave, 'box_world': _lower_box_world}
   if family not in lowerers:
     raise NotLoweredError(family)
   game = lowerers[family](engine, roles)

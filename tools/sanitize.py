@@ -3,6 +3,7 @@
 
     compute-sanitizer --tool memcheck  python tools/sanitize.py
     compute-sanitizer --tool racecheck python tools/sanitize.py
+    compute-sanitizer --tool memcheck  python tools/sanitize.py box_world   # that family alone
 
 Small batches (ragged last blocks, the 64 x 64 board, boards that are not multiples of 16 columns,
 auto-resets inside the run) so that out-of-bounds accesses and shared-memory
@@ -28,6 +29,7 @@ def main():
                                   scrolly_maze, warehouse_manager)
   from pycolab_b200.games.classics import chain_walk, cliff_walk, four_rooms
   rs = np.random.RandomState(0)
+  only = sys.argv[1] if len(sys.argv) > 1 else None     # e.g. `box_world`: that family alone
 
   def run(name, games, B, n_actions, steps=12, **kw):
     eng = batched.BatchedEngine(games, batch=B, **kw)
@@ -44,6 +46,17 @@ def main():
     print('ok %-28s B=%d launches=%d' % (name, B, eng.launch_count()))
     return eng
 
+  from pycolab_b200.games import box_world
+  pool = [box_world.make_game(12, (1, 2, 3, 4), (0, 1, 2, 3, 4), (0,), 1,
+                              random_state=np.random.RandomState(s), max_num_steps=6)
+          for s in range(5)]
+  run('box_world_step (rotation)', pool, 7, 8, steps=40, cycle_levels=True)
+  big = [box_world.make_game(30, (1, 2), (0, 1), (0,), 1, random_state=np.random.RandomState(s),
+                             max_num_steps=6) for s in range(3)]
+  run('box_world_step 32x32', big, 5, 8, steps=30, cycle_levels=True)
+  if only == 'box_world':
+    print('done')
+    return
   arts = [levels.scrolly_maze_level(5 + i, world_shape=(65, 65), board_shape=(20, 37))
           for i in range(2)]
   eng = run('scrolly_maze_step', [scrolly_maze.make_game(*a) for a in arts], 7, 6)
